@@ -11,7 +11,9 @@ streams of this rank.  Streams shard across ranks with no data-path collective (
     python bench.py [--gpus N] [--steps K] [--warmup W]             # CUDA arm
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # CPU reference arm
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definitions.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definitions.  --dump-outputs DIR (CUDA arm) also
+writes what the last timed step computed to DIR/<name>.npy (float64, see last_step_outputs); the inputs depend only
+on the arguments, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -184,6 +186,37 @@ def load_peaks():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_COV_STREAMS = 64
+
+
+def last_step_outputs(bt, batch, ids, counts):
+    """What a caller of the timed path holds after its last step, as float64 host arrays: the det -> track ids the
+    step returned (-1 past each stream's detection count), the counters all_reduce_counts returned, and the tracker's
+    per-stream counters and live tracks in track order (id, state, time since update, Kalman mean), padded past each
+    stream's track count with track_id -1 and zeros, so that every array is finite.  The Kalman covariances only for
+    a fixed, seeded sample of DUMP_COV_STREAMS streams (all of them would be 67 MB at C3)."""
+    import numpy as np
+    import torch
+    S, D = ids.shape
+    valid = torch.arange(D, device=ids.device)[None, :] < batch.count.to(ids.device)[:, None]
+    out = {"det_track_id": torch.where(valid, ids, -1).cpu().numpy(), "counts": counts.cpu().numpy()}
+    v = bt.host_view(["n_tracks", "order", "track_id", "state", "tsu", "mean", "counts"])
+    live = np.arange(v["order"].shape[1])[None, :] < v["n_tracks"][:, None]
+    slot = np.where(live, v["order"], 0)
+    rows = np.arange(S)[:, None]
+    for key, name in (("track_id", "track_id"), ("track_state", "state"), ("track_tsu", "tsu")):
+        out[key] = np.where(live, v[name][rows, slot], -1)
+    out["track_mean"] = np.where(live[..., None], v["mean"][rows, slot], 0.0)
+    out["stream_counts"] = v["counts"]
+    pick = np.sort(np.random.default_rng(0).choice(S, min(S, DUMP_COV_STREAMS), replace=False))
+    cov = bt.host_view(["cov"], streams=pick)["cov"]
+    out["track_cov"] = np.where(live[pick][..., None, None], cov[np.arange(len(pick))[:, None], slot[pick]], 0.0)
+    out["track_cov_streams"] = pick
+    out = {k: np.asarray(a, dtype=np.float64) for k, a in out.items()}
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20 and all(np.isfinite(a).all() for a in out.values())
+    return out
+
+
 def gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -233,8 +266,8 @@ def gpu_arm(args):
 
     # ---- main timed region: K ticks, stream chunks pipelined, counts reduced (+ NCCL) every tick
     def tick(b):
-        bt.step(b, join=False, reduce=True)
-        bt.all_reduce_counts(reduced=True, async_op=True)     # NCCL on its own stream: ranks do not rendezvous per tick
+        ids = bt.step(b, join=False, reduce=True)
+        return ids, bt.all_reduce_counts(reduced=True, async_op=True)   # NCCL on its own stream: no rendezvous per tick
 
     for b in frames[:W]:
         tick(b)
@@ -255,7 +288,7 @@ def gpu_arm(args):
     t0 = time.perf_counter()
     start.record()
     for b in frames[W:]:
-        tick(b)
+        last = tick(b)
     enq_ms = 1e3 * (time.perf_counter() - t0)      # host time to issue the K ticks ...
     st1 = bt.engine_stats()
     blocked_ms = st1[2] - st0[2]                   # ... of which blocked in the run-ahead throttle (pool polls: the host
@@ -268,6 +301,7 @@ def gpu_arm(args):
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    dump = last_step_outputs(bt, frames[-1], *last) if args.dump_outputs and rank == 0 else None
     ms = start.elapsed_time(end)
     state_bytes = bt.memory_bytes()
     # what the gallery kernel must move from HBM for the last tick, read from the work records k_gate wrote for it (one
@@ -417,6 +451,11 @@ def gpu_arm(args):
             "cpu_baseline": cpu,
             "configs": extras,
         }
+        if dump is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -456,7 +495,13 @@ def main():
     ap.add_argument("--no-graphs", action="store_true", help="A/B knob: the engine launches the tick's kernels plainly instead of replaying captured graphs")
     ap.add_argument("--match-warps", type=int, default=0, help="A/B knob: warps per stream in the matching kernel (0 = by size)")
     ap.add_argument("--chunks", type=int, default=2, help="stream chunks pipelined on separate CUDA streams")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; rank 0's streams)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs needs --impl cuda")
     set_workload(args.workload)
     args.warmup = max(args.warmup, 3) if args.impl == "cuda" else args.warmup
     if args.impl == "reference":
