@@ -305,11 +305,15 @@ DD_HD bool dd_yolo_row(const Row& row, const DDYoloParams& p, const unsigned cha
     const float obj = row(4);
     float best = dd_mulf(row(5), obj);
     int bi = 0;
+    bool nan = best != best;
     for (int c = 1; c < p.nc; ++c) {
         const float v = dd_mulf(row(5 + c), obj);
         if (v > best) { best = v; bi = c; }              // np.argmax: first maximum wins
+        nan = nan || v != v;
     }
-    if (!(best >= p.thr)) return false;                  // yolov5.py:130
+    // np.argmax returns the first NaN when there is one, and a NaN score fails the threshold: a NaN product anywhere
+    // in the row drops it, even when another class passes
+    if (nan || !(best >= p.thr)) return false;           // yolov5.py:130
     if (!wanted[bi]) return false;                       // yolov5.py:139
     const float cx = row(0), cy = row(1), w = row(2), h = row(3);
     const float hx = dd_divf(w, 2.0f), hy = dd_divf(h, 2.0f);

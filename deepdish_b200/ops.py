@@ -30,6 +30,24 @@ def _need_cuda(t):
         raise RuntimeError("deepdish_b200 operators run on CUDA tensors only (no CPU fallback)")
 
 
+def _arg(t, name, dtype, shape, device):
+    """The kernels read `t` as a dense row-major array of `dtype` on `device`: anything else (a slice, a
+    transposed view, another dtype or device, other extents) would be silently misread.  shape: ints, None = any."""
+    if not isinstance(t, torch.Tensor):
+        raise ValueError("%s must be a torch.Tensor" % name)
+    dtypes = dtype if isinstance(dtype, tuple) else (dtype,)
+    if t.dtype not in dtypes:
+        raise ValueError("%s must be %s, got %s" % (name, " or ".join(str(d) for d in dtypes), t.dtype))
+    if t.device != device:
+        raise ValueError("%s must be on %s, got %s" % (name, device, t.device))
+    if t.dim() != len(shape) or any(s is not None and s != n for s, n in zip(shape, t.shape)):
+        raise ValueError("%s must have shape [%s], got %s" % (
+            name, ",".join("*" if s is None else str(s) for s in shape), list(t.shape)))
+    if not t.is_contiguous():
+        raise ValueError("%s must be contiguous" % name)
+    return t
+
+
 # ------------------------------------------------------------------------------------- Kalman
 def kalman_initiate(xyah):
     """KalmanFilter.initiate (kalman_filter.py:55-86).  xyah f64 [n,4] -> mean [n,8], cov [n,8,8]."""
@@ -161,12 +179,18 @@ def nms(boxes, scores, counts, max_overlap, out=None):
     boxes f64 [b,nmax,4] tlwh, scores f32 [b,nmax], counts i32 [b] -> keep i32 [b,nmax], nkeep i32 [b].
     out = (keep, nkeep) reuses caller buffers (entries past nkeep are then left untouched)."""
     _need_cuda(boxes)
-    b, nmax = scores.shape
+    dev = boxes.device
+    _arg(boxes, "boxes", torch.float64, (None, None, 4), dev)
+    b, nmax = boxes.shape[:2]
+    _arg(scores, "scores", torch.float32, (b, nmax), dev)
+    _arg(counts, "counts", torch.int32, (b,), dev)
     if out is None:
-        keep = torch.full((b, nmax), -1, dtype=torch.int32, device=boxes.device)
-        nkeep = torch.zeros((b,), dtype=torch.int32, device=boxes.device)
+        keep = torch.full((b, nmax), -1, dtype=torch.int32, device=dev)
+        nkeep = torch.zeros((b,), dtype=torch.int32, device=dev)
     else:
         keep, nkeep = out
+        _arg(keep, "out keep", torch.int32, (b, nmax), dev)
+        _arg(nkeep, "out nkeep", torch.int32, (b,), dev)
     _lib.check(_lib.lib().dd_nms(boxes.data_ptr(), scores.data_ptr(), counts.data_ptr(), b, nmax,
                                  float(max_overlap), keep.data_ptr(), nkeep.data_ptr(), _stream(boxes.device)),
                "dd_nms")
@@ -177,7 +201,10 @@ def box_filter(boxes, counts=None, frame_size=(640, 480)):
     """The pre-NMS box filter of Pipeline.detect_objects (deepdish.py:941-960) for b frames of float tlwh boxes.
     boxes f64 [b,nmax,4], counts i32 [b] or None -> (tlwh f64 [b,nmax,4] integer-valued, index i32 [b,nmax], count i32 [b])."""
     _need_cuda(boxes)
+    _arg(boxes, "boxes", torch.float64, (None, None, 4), boxes.device)
     b, nmax = boxes.shape[:2]
+    if counts is not None:
+        _arg(counts, "counts", torch.int32, (b,), boxes.device)
     out = torch.zeros((b, nmax, 4), dtype=torch.float64, device=boxes.device)
     idx = torch.full((b, nmax), -1, dtype=torch.int32, device=boxes.device)
     cnt = torch.zeros((b,), dtype=torch.int32, device=boxes.device)
@@ -193,21 +220,20 @@ def yolo_decode(head, wanted_mask, score_thr=0.25, img_size=(640, 480), frame_si
     head f32 [b,na,5+nc] (or u8 with quant=(scale, zero_point)); wanted_mask u8 [nc].
     Returns dict(tlwh f64 [b,ncap,4], score f32, cls i32, anchor i32, count i32 [b], flags i32 [b])."""
     _need_cuda(head)
+    dev = head.device
+    _arg(head, "head", (torch.float32, torch.uint8), (None, None, None), dev)
     b, na, rw = head.shape
     nc = rw - 5
-    dev = head.device
+    _arg(wanted_mask, "wanted_mask", torch.uint8, (nc,), dev)
+    spec = dict(tlwh=(torch.float64, (b, ncap, 4)), score=(torch.float32, (b, ncap)), cls=(torch.int32, (b, ncap)),
+                anchor=(torch.int32, (b, ncap)), count=(torch.int32, (b,)), flags=(torch.int32, (b,)))
     if out is None:      # pass the previous result back as `out` to reuse its buffers (rows past count are stale)
-        out = dict(tlwh=torch.zeros((b, ncap, 4), dtype=torch.float64, device=dev),
-                   score=torch.zeros((b, ncap), dtype=torch.float32, device=dev),
-                   cls=torch.zeros((b, ncap), dtype=torch.int32, device=dev),
-                   anchor=torch.zeros((b, ncap), dtype=torch.int32, device=dev),
-                   count=torch.zeros((b,), dtype=torch.int32, device=dev),
-                   flags=torch.zeros((b,), dtype=torch.int32, device=dev))
+        out = {k: torch.zeros(s, dtype=dt, device=dev) for k, (dt, s) in spec.items()}
+    for k, (dt, s) in spec.items():
+        _arg(out[k], "out[%r]" % k, dt, s, dev)
     is_u8 = head.dtype == torch.uint8
     if is_u8 and quant is None:
         raise ValueError("u8 head needs quant=(scale, zero_point)")
-    if not is_u8 and head.dtype != torch.float32:
-        raise ValueError("head must be float32 or uint8")
     scale, zp = quant if is_u8 else (1.0, 0)
     _lib.check(_lib.lib().dd_yolo_decode(head.data_ptr(), 1 if is_u8 else 0, float(scale), int(zp), b, na, nc,
                                          wanted_mask.data_ptr(), float(score_thr), int(img_size[0]),
@@ -248,15 +274,23 @@ def ssd_decode(raw_boxes, raw_scores, anchors, class_to_label, conf_thr=0.5, nms
     [b,na,ncls], anchors f32 [na,4], class_to_label i32 [ncls-1].
     Returns dict(tlwh f64 [b,ncap,4], score f32, label i32, count i32 [b], flags i32 [b])."""
     _need_cuda(raw_boxes)
-    b, na, _ = raw_boxes.shape
-    ncls = raw_scores.shape[2]
     dev = raw_boxes.device
+    _arg(raw_boxes, "raw_boxes", torch.float32, (None, None, 4), dev)
+    b, na, _ = raw_boxes.shape
+    _arg(raw_scores, "raw_scores", torch.float32, (b, na, None), dev)
+    ncls = raw_scores.shape[2]
+    _arg(anchors, "anchors", torch.float32, (na, 4), dev)
+    _arg(class_to_label, "class_to_label", torch.int32, (ncls - 1,), dev)
+    spec = dict(tlwh=(torch.float64, (b, ncap, 4)), score=(torch.float32, (b, ncap)), label=(torch.int32, (b, ncap)),
+                count=(torch.int32, (b,)), flags=(torch.int32, (b,)))
     if out is None:
         out = dict(tlwh=torch.zeros((b, ncap, 4), dtype=torch.float64, device=dev),
                    score=torch.zeros((b, ncap), dtype=torch.float32, device=dev),
                    label=torch.full((b, ncap), -1, dtype=torch.int32, device=dev),
                    count=torch.zeros((b,), dtype=torch.int32, device=dev),
                    flags=torch.zeros((b,), dtype=torch.int32, device=dev))
+    for k, (dt, s) in spec.items():
+        _arg(out[k], "out[%r]" % k, dt, s, dev)
     _lib.check(_lib.lib().dd_ssd_decode(raw_boxes.data_ptr(), raw_scores.data_ptr(), anchors.data_ptr(), b, na, ncls,
                                         class_to_label.data_ptr(), float(conf_thr), float(nms_iou),
                                         int(img_size[0]), int(img_size[1]), int(frame_size[0]), int(frame_size[1]),
@@ -272,9 +306,16 @@ def tflite_postprocess(op_boxes, op_classes, op_scores, op_count, list_ok, wante
     op_boxes f32 [b,n,4], op_classes f32 [b,n], op_scores f32 [b,n], op_count i32 [b]; list_ok / wanted u8 [n_labels].
     Returns dict(tlwh f64 [b,ncap,4], score f32, label i32, count i32 [b], flags i32 [b])."""
     _need_cuda(op_boxes)
-    b, n, _ = op_boxes.shape
-    ncap = n if ncap is None else ncap
     dev = op_boxes.device
+    _arg(op_boxes, "op_boxes", torch.float32, (None, None, 4), dev)
+    b, n, _ = op_boxes.shape
+    _arg(op_classes, "op_classes", torch.float32, (b, n), dev)
+    _arg(op_scores, "op_scores", torch.float32, (b, n), dev)
+    _arg(op_count, "op_count", torch.int32, (b,), dev)
+    _arg(list_ok, "list_ok", torch.uint8, (None,), dev)
+    _arg(wanted, "wanted", torch.uint8, list_ok.shape, dev)
+    ncap = n if ncap is None else ncap
+
     out = dict(tlwh=torch.zeros((b, ncap, 4), dtype=torch.float64, device=dev),
                score=torch.zeros((b, ncap), dtype=torch.float32, device=dev),
                label=torch.full((b, ncap), -1, dtype=torch.int32, device=dev),

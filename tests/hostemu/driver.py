@@ -106,7 +106,7 @@ def ssd_post(sel_box, sel_cls, sel_score, class_to_label, conf_thr=0.5, nms_iou=
     return tl[:k], sc[:k], lb[:k]
 
 
-def yolo3(maps, anchors, nc, wanted_mask, thr, image, net, ncap=256):
+def yolo3(maps, anchors, nc, wanted_mask, thr, image, net, ncap=256, nms_thresh=0.5):
     m = [np.ascontiguousarray(x, np.float32) for x in maps]
     grids = np.array([x.shape[0] for x in m], np.int32)
     anch = np.ascontiguousarray(anchors, np.int32).reshape(-1)
@@ -114,7 +114,7 @@ def yolo3(maps, anchors, nc, wanted_mask, thr, image, net, ncap=256):
     box = np.zeros((ncap, 4)); sc = np.zeros(ncap, np.float32); lb = np.zeros(ncap, np.int32); fl = np.zeros(1, np.int32)
     emu().ddh_yolo3.argtypes = [ctypes.c_void_p] * 5 + [ctypes.c_int, ctypes.c_void_p, ctypes.c_float, ctypes.c_double] + \
         [ctypes.c_int] * 5 + [ctypes.c_void_p] * 4
-    k = emu().ddh_yolo3(_p(m[0]), _p(m[1]), _p(m[2]), _p(grids), _p(anch), nc, _p(wm), thr, 0.5, image[0], image[1],
+    k = emu().ddh_yolo3(_p(m[0]), _p(m[1]), _p(m[2]), _p(grids), _p(anch), nc, _p(wm), thr, nms_thresh, image[0], image[1],
                         net[0], net[1], ncap, _p(box), _p(sc), _p(lb), _p(fl))
     return box[:k], sc[:k], lb[:k], int(fl[0])
 

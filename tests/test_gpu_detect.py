@@ -61,6 +61,7 @@ def test_yolo_u8_head_and_overflow_flag():
         assert n == len(kept) and n > 20
         np.testing.assert_array_equal(o["tlwh"][f, :n], ib.astype(np.float64))
         np.testing.assert_array_equal(o["score"][f, :n], score[kept])
+        np.testing.assert_array_equal(o["cls"][f, :n], cls[kept])          # u8 ties for the top class: first one wins
         np.testing.assert_array_equal(o["anchor"][f, :n], anchor[kept])
     small = ops.yolo_decode(torch.from_numpy(q).cuda(), mask, 0.25, (640, 480), (640, 480), ncap=8, quant=(scale, zp))
     assert int(small["flags"].cpu()[0]) & _lib.FLAG_DET_OVERFLOW          # never silently truncated
