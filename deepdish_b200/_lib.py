@@ -128,14 +128,7 @@ def lib():
         "dd_event_destroy": [_vp],
         "dd_event_elapsed_ms": [_vp, _vp, ctypes.POINTER(ctypes.c_float)],
         "dd_event_record": [_vp, _vp],
-        "dd_event_query": [_vp],
-        "dd_event_synchronize": [_vp],
-        "dd_tracker_pool_poll": [_vp, cfgp, _vp, _vp, _vp],
         "dd_tracker_countline": [_vp, cfgp, _vp, _i32, _vp],
-        "dd_tracker_tick": [_vp, cfgp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp],
-        "dd_tracker_tick_profiled": [_vp, cfgp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, ctypes.POINTER(_vp)],
-        "dd_tracker_tick_ragged": [_vp, cfgp, _vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64,
-                                   _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp],
         "dd_unpack_detections": [_vp, _i32, _i32, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64,
                                  _vp, _vp, _vp, _vp, _vp, _vp],
         "dd_tracker_count_reduce": [_vp, cfgp, _vp, _vp],

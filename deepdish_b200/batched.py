@@ -62,8 +62,6 @@ class _Chunk:
         self.cfg.n_segs = n_segs
         self._bind()
         self.done = torch.cuda.Event()
-        self.staging = None
-        self.poll = None              # (pinned copy of pool_ctl[:4], event) of the latest tick
 
     def _alloc_seg(self):
         k = len(self.segs)
@@ -111,7 +109,6 @@ class _Chunk:
                 t[:, :, :pt].copy_(old[name])
             else:
                 t.copy_(old[name])
-        self.poll = None
 
 
 class _CatView:
@@ -183,8 +180,6 @@ class BatchedTracker:
         self.partial_counts = torch.zeros((2, n_chunks, C, 4), dtype=torch.int64, device=self.device)
         self.total_counts = torch.zeros((C, 4), dtype=torch.int64, device=self.device)
         self._tick = 0
-        self._sum_done = [None, None]
-        self._last_sum = None
         self._aux = torch.cuda.Stream(device=self.device) if n_chunks > 1 else None
         self._poll_pool = any(len(c.segs) * c.cfg.seg_pages < self._worst_pages(c) for c in self.chunks) or budget is None
         self._engine = None           # native tick engine (csrc/dd_engine.cu), created at the first step()
@@ -227,8 +222,10 @@ class BatchedTracker:
             pass
 
     def _enter(self, mode):
-        """Ticks can be issued through the engine ("eng") or call by call from Python ("py": update(), step_host(), the
-        kernel-timeline mode).  Each side tracks its own cross-tick events, so a switch re-orders every stream first."""
+        """Work is issued through the engine ("eng": step(), step_host_packed()) or call by call from Python ("py":
+        predict(), update(), countline(), reduce_counts()).  A switch re-orders every stream first: dd_engine_step_host
+        does not fork from the caller's stream, and the engine's count summation on the auxiliary stream writes
+        total_counts, which reduce_counts() writes on the caller's stream."""
         if mode == self._mode:
             return
         if self._mode is not None and len(self.chunks) > 1:
@@ -258,29 +255,12 @@ class BatchedTracker:
 
     UPLOAD_BUFFERS = 2    # device blobs a chunk's ragged host batches rotate through (step_host_packed); 3 and 4 measured
                           # slower end to end (0.587 / 0.603 vs 0.569 ms per tick): the link, not the buffer depth, is the bound
-    POLL_EVERY = 2        # ticks between polls of the pool counters (the forecast covers 8 appends ahead)
-
-    def _post_tick(self, c, st):
-        """After a chunk's tick was enqueued on stream ``st``: every POLL_EVERY ticks copy its pool counters to
-        pinned memory (dd_tracker_pool_poll; no host synchronisation) so that ``maintain`` can grow the pool ahead
-        of need."""
-        if not self._poll_pool or self._tick % self.POLL_EVERY:
-            return
-        if c.poll is None:
-            ev = ctypes.c_void_p()
-            _lib.check(self.lib.dd_event_create(ctypes.byref(ev)), "dd_event_create")
-            c.poll = [torch.zeros(4, dtype=torch.int32).pin_memory(), ev, -1, True]    # host copy, event, tick, seen
-        host, ev, tick, seen = c.poll
-        if tick >= 0 and not seen and self.lib.dd_event_query(ev) != 1:
-            return                                    # the previous poll is still in flight: keep it
-        _lib.check(self.lib.dd_tracker_pool_poll(c.state, c.cfgp, host.data_ptr(), ev, ctypes.c_void_p(st.cuda_stream)),
-                   "dd_tracker_pool_poll")
-        c.poll[2], c.poll[3] = self._tick, False
+    POLL_EVERY = 2        # ticks between the engine's polls of the pool counters (the forecast covers 8 appends ahead)
 
     def maintain(self, wait=False):
-        """Grow gallery storage ahead of need, from the latest poll of every chunk's pool counters (``wait=True``:
-        from the state right now, synchronising).  A poll that is 3 ticks old is waited for, so the host never runs
-        further ahead of the device than the 8-append forecast covers.
+        """Grow gallery storage ahead of need, from the engine's latest poll of every chunk's pool counters
+        (``wait=True``: from the state right now, synchronising).  A poll that is 3 ticks old is waited for, so the host
+        never runs further ahead of the device than the 8-append forecast covers.
         Pool: segments are attached until the free pages cover the forecast (pages the live tracks can take within
         their next 8 appends) plus one page per detection slot (new tracks).  Unbounded galleries: the page table is doubled when the
         longest gallery is within 128 rows of its capacity."""
@@ -289,22 +269,13 @@ class BatchedTracker:
             if wait:
                 st.synchronize()
                 ctl = c.v["pool_ctl"][:4].cpu()
-            elif self._mode == "eng":
-                if self._engine is None:
-                    continue
+            elif self._mode == "eng" and self._engine is not None:
                 out, tick = (ctypes.c_int32 * 4)(), ctypes.c_int64(-1)
                 _lib.check(self.lib.dd_engine_pool_latest(self._engine, i, 3, out, ctypes.byref(tick)), "dd_engine_pool_latest")
                 if tick.value < 0 or tick.value == getattr(c, "eng_poll_seen", -1):
                     continue
                 c.eng_poll_seen = tick.value
                 ctl = out
-            elif c.poll is not None and c.poll[2] >= 0 and not c.poll[3]:
-                if self.lib.dd_event_query(c.poll[1]) != 1:
-                    if self._tick - c.poll[2] < 3:
-                        continue
-                    _lib.check(self.lib.dd_event_synchronize(c.poll[1]), "dd_event_synchronize")
-                ctl = c.poll[0]
-                c.poll[3] = True
             else:
                 continue
             free, attached, longest, forecast = int(ctl[0]), int(ctl[1]), int(ctl[2]), int(ctl[3])
@@ -347,11 +318,6 @@ class BatchedTracker:
             for t in tensors:
                 t.record_stream(c.stream)
 
-    def _mark(self):
-        if len(self.chunks) > 1:
-            for c in self.chunks:
-                c.done.record(c.stream)
-
     def join(self):
         """Make the caller's current stream wait for all chunk streams and for the count summation (no host
         synchronisation)."""
@@ -361,8 +327,6 @@ class BatchedTracker:
         for c in self.chunks:
             c.done.record(c.stream)
             cur.wait_event(c.done)
-        if self._last_sum is not None:
-            cur.wait_event(self._last_sum)
         if self._engine is not None:
             _lib.check(self.lib.dd_engine_join(self._engine, ctypes.c_void_p(cur.cuda_stream)), "dd_engine_join")
 
@@ -398,16 +362,19 @@ class BatchedTracker:
         """Tracker.update for every stream (tracker.py:59-93).
 
         tlwh f64 [S,Dmax,4], conf f32 [S,Dmax], label i32 [S,Dmax], feat f32 [S,Dmax,128], count i32 [S]
-        -- device tensors, padded.  Returns det_track_id i32 [S,Dmax] (device; -1 = padding)."""
+        -- device tensors, padded.  Returns det_track_id i32 [S,Dmax] (device; -1 = padding).
+
+        When the gallery storage can grow (a pool smaller than the worst case, or unbounded galleries), the update first
+        grows it from the exact counters (``maintain(wait=True)``): the call blocks until the work already enqueued on
+        the tracker's streams has run."""
         self._check_batch(tlwh, conf, label, feat, count)
         self._enter("py")
         if self._poll_pool:
-            self.maintain()
+            self.maintain(wait=True)
         self._fork((tlwh, conf, label, feat, count))
         for c in self.chunks:
             p = self._ptrs(c, tlwh, conf, label, feat, count, self.det_track_id)
             _lib.check(self.lib.dd_tracker_update(c.state, c.cfgp, *p, self._sp(c)), "dd_tracker_update")
-            self._post_tick(c, c.stream if c.stream is not None else self._cur())
         self.join()
         return self.det_track_id
 
@@ -449,8 +416,6 @@ class BatchedTracker:
         only enqueues (call join())."""
         tlwh, conf, label, feat, count = batch.tlwh, batch.conf, batch.label, batch.feat, batch.count
         self._check_batch(tlwh, conf, label, feat, count)
-        if getattr(self, "_timeline", None):
-            return self._step_py(batch, join, reduce)
         self._enter("eng")
         if self._poll_pool:
             self.maintain()
@@ -466,100 +431,7 @@ class BatchedTracker:
             self.join()
         return self.det_track_id
 
-    def _step_py(self, batch, join=True, reduce=False):
-        """step() issued call by call from Python (one dd_tracker_tick per chunk): the kernel-timeline mode of
-        benchmarks/timeline.py, which needs events between the kernels."""
-        tlwh, conf, label, feat, count = batch.tlwh, batch.conf, batch.label, batch.feat, batch.count
-        self._enter("py")
-        if self._poll_pool:
-            self.maintain()
-        self._fork((tlwh, conf, label, feat, count))
-        par = self._tick & 1
-        multi = len(self.chunks) > 1
-        if reduce and multi and self._sum_done[par] is not None:
-            for c in self.chunks:              # partial_counts[par] of tick-2 must have been summed
-                c.stream.wait_event(self._sum_done[par])
-        for i, c in enumerate(self.chunks):
-            p = self._ptrs(c, tlwh, conf, label, feat, count, self.det_track_id)
-            out = self.partial_counts[par, i].data_ptr() if reduce else None
-            self._tick_call(c, p, out, self._sp(c))
-            self._post_tick(c, c.stream if c.stream is not None else self._cur())
-        self._mark()
-        if reduce:
-            self._sum_partials(par)
-        self._tick += 1
-        if join:
-            self.join()
-        return self.det_track_id
-
-    def _tick_call(self, c, p, out, sp):
-        ev = self._timeline.pop(0) if getattr(self, "_timeline", None) else None
-        if ev is not None:         # kernel-timeline mode (benchmarks/timeline.py): 8 events around this chunk's kernels
-            _lib.check(self.lib.dd_tracker_tick_profiled(c.state, c.cfgp, *p, self._line_ptr(c), self.line_per_stream,
-                                                         out, sp, ev), "dd_tracker_tick_profiled")
-            return
-        _lib.check(self.lib.dd_tracker_tick(c.state, c.cfgp, *p, self._line_ptr(c), self.line_per_stream, out, sp),
-                   "dd_tracker_tick")
-
-    def _sum_partials(self, par):
-        """Sum the chunks' partial counters of this tick into total_counts.  With several chunks this runs on the
-        tracker's own auxiliary stream, NOT on the caller's: the caller's stream must not wait for every chunk each
-        tick, or the next tick's fork event would serialise the chunks tick by tick and nothing would overlap
-        across tick boundaries.  total_counts is valid on the caller's stream after join()."""
-        if len(self.chunks) == 1:
-            torch.sum(self.partial_counts[par], dim=0, out=self.total_counts)
-            return
-        with torch.cuda.stream(self._aux):
-            for c in self.chunks:
-                self._aux.wait_event(c.done)
-            torch.sum(self.partial_counts[par], dim=0, out=self.total_counts)
-            self._sum_done[par] = self._last_sum = self._aux.record_event()
-
-    def step_host(self, host_batch, out_ids_host=None):
-        """End-to-end tick from a pinned HOST batch: per chunk and on the chunk's stream, H2D copy of its
-        slice into a staging buffer, the tick, the partial count reduction and (optionally) the D2H copy
-        of its det->track ids into the pinned ``out_ids_host``.  Returns total_counts (device, summed on the
-        caller's stream)."""
-        D = self.max_dets
-        self._enter("py")
-        if self._poll_pool:
-            self.maintain()
-        par = self._tick & 1
-        multi = len(self.chunks) > 1
-        if multi and self._sum_done[par] is not None:
-            for c in self.chunks:
-                c.stream.wait_event(self._sum_done[par])
-        src = (host_batch.tlwh, host_batch.conf, host_batch.label, host_batch.feat, host_batch.count)
-        for i, c in enumerate(self.chunks):
-            n = c.hi - c.lo
-            st = c.stream if multi else self._cur()
-            with torch.cuda.stream(st):
-                for dst, s in zip(self._staging(c), src):
-                    dst.copy_(s[c.lo:c.hi], non_blocking=True)
-                t, cf, lb, ft, ct = c.staging
-                ids = self.det_track_id[c.lo:c.hi]
-                self._tick_call(c, (t.data_ptr(), cf.data_ptr(), lb.data_ptr(), ft.data_ptr(), ct.data_ptr(),
-                                    ids.data_ptr()), self.partial_counts[par, i].data_ptr(),
-                                ctypes.c_void_p(st.cuda_stream))
-                if out_ids_host is not None:
-                    out_ids_host[c.lo:c.hi].copy_(ids, non_blocking=True)
-            self._post_tick(c, st)
-        self._mark()
-        self._sum_partials(par)
-        self._tick += 1
-        return self.total_counts
-
     # ------------------------------------------------------------------------------------------
-    def _staging(self, c):
-        if c.staging is None:
-            n, D = c.hi - c.lo, self.max_dets
-            c.staging = (torch.empty((n, D, 4), dtype=torch.float64, device=self.device),
-                         torch.empty((n, D), dtype=torch.float32, device=self.device),
-                         torch.empty((n, D), dtype=torch.int32, device=self.device),
-                         torch.empty((n, D, 128), dtype=torch.float32, device=self.device),
-                         torch.empty((n,), dtype=torch.int32, device=self.device))
-        return c.staging
-
     def _staging_small(self, c):
         if getattr(c, "staging_small", None) is None:
             n, D = c.hi - c.lo, self.max_dets
@@ -627,27 +499,20 @@ class BatchedTracker:
         return self.total_counts
 
     def reduce_counts(self):
-        """Sum the per-stream counters -> i64 [C,4] (pos, neg, int, del per label), this GPU only."""
+        """Sum the per-stream counters -> i64 [C,4] (pos, neg, int, del per label), this GPU only.  Runs on the caller's
+        stream, behind every chunk."""
         self._enter("py")
-        self._fork()
-        par = self._tick & 1
-        multi = len(self.chunks) > 1
-        if multi and self._sum_done[par] is not None:
-            for c in self.chunks:
-                c.stream.wait_event(self._sum_done[par])
+        self.join()
+        sp = ctypes.c_void_p(self._cur().cuda_stream)
         for i, c in enumerate(self.chunks):
-            _lib.check(self.lib.dd_tracker_count_reduce(c.state, c.cfgp, self.partial_counts[par, i].data_ptr(),
-                                                        self._sp(c)), "dd_tracker_count_reduce")
-        self._mark()
-        self._sum_partials(par)
-        self._tick += 1
-        if self._last_sum is not None:
-            self._cur().wait_event(self._last_sum)
+            _lib.check(self.lib.dd_tracker_count_reduce(c.state, c.cfgp, self.partial_counts[0, i].data_ptr(), sp),
+                       "dd_tracker_count_reduce")
+        torch.sum(self.partial_counts[0], dim=0, out=self.total_counts)
         return self.total_counts
 
     def all_reduce_counts(self, reduced=False, async_op=False):
         """[C,4] counters summed over streams and, over NCCL, ranks (the path's only collective).
-        reduced=True: total_counts already holds this tick's local sum (step(reduce=True) / step_host).
+        reduced=True: total_counts already holds this tick's local sum (step(reduce=True) / step_host_packed).
         async_op=True: the all-reduce runs on NCCL's own stream on a copy of the counters (two alternating buffers)
         and the caller's stream is not made to wait, so ranks do not rendezvous every tick; the returned tensor is
         valid after wait_counts()."""
@@ -667,7 +532,9 @@ class BatchedTracker:
             self._ar_turn = 0
         k = self._ar_turn
         self._ar_turn ^= 1
-        side = self._aux if self._aux is not None else self._cur()      # the stream total_counts is produced on
+        # the stream total_counts is produced on: the engine sums several chunks on the auxiliary stream, reduce_counts()
+        # on the caller's
+        side = self._aux if self._mode == "eng" and self._aux is not None else self._cur()
         with torch.cuda.stream(side):
             if self._ar_work[k] is not None:
                 self._ar_work[k].wait()
@@ -677,9 +544,8 @@ class BatchedTracker:
         return self._ar_buf[k]
 
     def _wait_sum(self):
-        """The caller's stream waits for the latest count summation (Python-issued or the engine's)."""
-        if self._last_sum is not None:
-            self._cur().wait_event(self._last_sum)
+        """The caller's stream waits for the engine's latest count summation (reduce_counts() sums on the caller's
+        stream)."""
         if self._engine is not None:
             _lib.check(self.lib.dd_engine_wait_counts(self._engine, ctypes.c_void_p(self._cur().cuda_stream)),
                        "dd_engine_wait_counts")
@@ -754,13 +620,10 @@ class BatchedTracker:
             for (a, h), (pa, ph) in zip(c.segs, pool):
                 a.copy_(pa.to(self.device))
                 h.copy_(ph.to(self.device))
-            c.poll = None
             c.eng_poll_seen = -1
             self._rebind(c)
         self.total_counts.copy_(sd["total_counts"].to(self.device))
         self._tick = int(sd["tick"])
-        self._sum_done = [None, None]
-        self._last_sum = None
         torch.cuda.synchronize(self.device)
 
     def host_view(self, names=None, streams=None):

@@ -474,21 +474,19 @@ static int dd_update_impl(void* state, const dd_tracker_config* cfg, const DDTic
     return DD_OK;
 }
 
-// out_counts: by value, or (captured tick) `indirect` = read args->out_counts from the blob
-static int dd_tick_tail(void* state, const dd_tracker_config* cfg, const double* line, int line_per_stream,
-                        int64_t* out_counts, bool indirect, cudaStream_t st, cudaEvent_t* ev = nullptr) {
+// reduce (captured tick): the count reduction into the tick's out_counts, read from the blob's tick_args words
+static int dd_tick_tail(void* state, const dd_tracker_config* cfg, const double* line, int line_per_stream, bool reduce,
+                        cudaStream_t st) {
     DDView V;
     int rc = dd_make_view(state, cfg, &V);
     if (rc != DD_OK) return rc;
     dd_launch(k_countline, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
     DD_CHECK_LAUNCH();
-    if (ev) cudaEventRecord(ev[6], st);
-    if (out_counts || indirect) {
-        dd_launch(k_count_reduce, V.C * 4, 256, 0, st, (const long long*)V.counts, V.S, V.C * 4, (long long*)out_counts,
-                  indirect ? V.targs : (const DDTickArgs*)nullptr);
+    if (reduce) {
+        dd_launch(k_count_reduce, V.C * 4, 256, 0, st, (const long long*)V.counts, V.S, V.C * 4, (long long*)nullptr,
+                  (const DDTickArgs*)V.targs);
         DD_CHECK_LAUNCH();
     }
-    if (ev) cudaEventRecord(ev[7], st);
     return DD_OK;
 }
 
@@ -516,7 +514,7 @@ int dd_capture_tick(void* state, const dd_tracker_config* cfg, int ragged, int r
         const int rc = dd_update_impl(state, cfg, A, st, nullptr, true, parts);
         if (rc != DD_OK) return rc;
     }
-    if (parts & DD_PART_TAIL) return dd_tick_tail(state, cfg, line, line_per_stream, nullptr, reduce != 0, st);
+    if (parts & DD_PART_TAIL) return dd_tick_tail(state, cfg, line, line_per_stream, reduce != 0, st);
     return DD_OK;
 }
 #ifdef DD_GS_VARIANTS
@@ -683,69 +681,10 @@ int dd_event_record(void* ev, void* stream) {
     return cudaEventRecord((cudaEvent_t)ev, (cudaStream_t)stream) == cudaSuccess ? DD_OK : DD_ERR_CUDA;
 }
 
-int dd_event_query(void* ev) {
-    const cudaError_t e = cudaEventQuery((cudaEvent_t)ev);
-    return e == cudaSuccess ? 1 : (e == cudaErrorNotReady ? 0 : DD_ERR_CUDA);
-}
-
-int dd_event_synchronize(void* ev) {
-    return cudaEventSynchronize((cudaEvent_t)ev) == cudaSuccess ? DD_OK : DD_ERR_CUDA;
-}
-
-int dd_tracker_pool_poll(void* state, const dd_tracker_config* cfg, int32_t* host_pinned4, void* done_event,
-                         void* stream) {
-    DDView V;
-    int rc = dd_make_view(state, cfg, &V);
-    if (rc != DD_OK) return rc;
-    if (!host_pinned4) return DD_ERR_INVALID;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (cudaMemcpyAsync(host_pinned4, V.pool_ctl, 4 * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess) return DD_ERR_CUDA;
-    if (done_event && cudaEventRecord((cudaEvent_t)done_event, st) != cudaSuccess) return DD_ERR_CUDA;
-    return DD_OK;
-}
-
 int dd_tracker_countline(void* state, const dd_tracker_config* cfg, const double* line,
                          int line_per_stream, void* stream) {
     if (!line) return DD_ERR_INVALID;
-    return dd_tick_tail(state, cfg, line, line_per_stream, nullptr, false, (cudaStream_t)stream);
-}
-
-int dd_tracker_tick(void* state, const dd_tracker_config* cfg, const double* det_tlwh,
-                    const float* det_conf, const int32_t* det_label, const float* det_feat,
-                    const int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                    int line_per_stream, int64_t* out_counts, void* stream) {
-    if (!line) return DD_ERR_INVALID;
-    const DDTickArgs in = dd_args_padded(det_tlwh, det_conf, det_label, det_feat, det_count, out_det_track_id);
-    const int rc = dd_update_impl(state, cfg, in, (cudaStream_t)stream, nullptr, true);
-    if (rc != DD_OK) return rc;
-    return dd_tick_tail(state, cfg, line, line_per_stream, out_counts, false, (cudaStream_t)stream);
-}
-
-int dd_tracker_tick_profiled(void* state, const dd_tracker_config* cfg, const double* det_tlwh,
-                             const float* det_conf, const int32_t* det_label, const float* det_feat,
-                             const int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                             int line_per_stream, int64_t* out_counts, void* stream, void* const* host_events8) {
-    if (!line || !host_events8) return DD_ERR_INVALID;
-    cudaEvent_t ev[8];
-    for (int i = 0; i < 8; ++i) ev[i] = (cudaEvent_t)host_events8[i];
-    const DDTickArgs in = dd_args_padded(det_tlwh, det_conf, det_label, det_feat, det_count, out_det_track_id);
-    const int rc = dd_update_impl(state, cfg, in, (cudaStream_t)stream, ev, true);
-    if (rc != DD_OK) return rc;
-    return dd_tick_tail(state, cfg, line, line_per_stream, out_counts, false, (cudaStream_t)stream, ev);
-}
-
-int dd_tracker_tick_ragged(void* state, const dd_tracker_config* cfg, const void* blob, int64_t off_tlwh,
-                           int64_t off_conf, int64_t off_label, int64_t off_feat, double* det_tlwh, float* det_conf,
-                           int32_t* det_label, int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                           int line_per_stream, int64_t* out_counts, void* stream) {
-    if (!line || !blob) return DD_ERR_INVALID;
-    if ((off_tlwh & 7) || (off_conf & 3) || (off_label & 3) || (off_feat & 15) || ((uintptr_t)blob & 15)) return DD_ERR_INVALID;
-    DDTickArgs in = dd_args_padded(det_tlwh, det_conf, det_label, nullptr, det_count, out_det_track_id);
-    in.blob = (const unsigned char*)blob;
-    in.off_tlwh = off_tlwh; in.off_conf = off_conf; in.off_label = off_label; in.off_feat = off_feat;
-    const int rc = dd_update_impl(state, cfg, in, (cudaStream_t)stream, nullptr, true);
-    if (rc != DD_OK) return rc;
-    return dd_tick_tail(state, cfg, line, line_per_stream, out_counts, false, (cudaStream_t)stream);
+    return dd_tick_tail(state, cfg, line, line_per_stream, false, (cudaStream_t)stream);
 }
 
 int dd_unpack_detections(const void* blob, int32_t n_streams, int32_t max_dets, int64_t off_tlwh, int64_t off_conf,

@@ -233,8 +233,6 @@ class Tracker:
         self.last_detection_track_ids = self._ids_host[:n].numpy().copy()
         self._stale = True
         self.metric.samples = _LazySamples(self)
-        if bt._poll_pool:
-            bt.maintain(wait=True)                  # unbounded galleries (nn_budget=None): grow pool / page table
         if flags.value:
             bt.check()                              # raises with the reason
         if self._late_features:

@@ -9,7 +9,7 @@ batched equivalent on the wire between host and device is ONE contiguous blob pe
     (pad to 16 bytes)
     f32 feat[N][128]
 
-holding only the detections that exist -- what ``dd_tracker_tick_ragged`` / ``dd_unpack_detections`` read
+holding only the detections that exist -- what ``dd_engine_step_host`` / ``dd_unpack_detections`` read
 (include/deepdish_b200.h).  ``section_offsets`` is the single definition of the layout.
 """
 import numpy as np

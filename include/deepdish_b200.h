@@ -213,35 +213,13 @@ int dd_event_create(void** host_out);
 int dd_event_destroy(void* ev);
 int dd_event_elapsed_ms(void* start, void* end, float* host_ms);   /* both events must have completed */
 int dd_event_record(void* ev, void* stream);
-int dd_event_query(void* ev);          /* 1 = completed, 0 = not yet, negative = error */
-int dd_event_synchronize(void* ev);
-
-/* Copy the pool counters pool_ctl[0..3] (free pages, pages attached, longest gallery, page-demand forecast) to
- * PINNED host memory on `stream` and record done_event (may be NULL) behind the copy: no host synchronisation. */
-int dd_tracker_pool_poll(void* state, const dd_tracker_config* host_cfg, int32_t* host_pinned4, void* done_event,
-                         void* stream);
 
 /* Count-line step (deepdish.py:1035-1114 counting part, :1303-1312; tools/intersection.py:4-30).
  *   line f64 [S,4] (x1,y1,x2,y2 per stream) or, with line_per_stream = 0, one f64[4] for all streams. */
 int dd_tracker_countline(void* state, const dd_tracker_config* host_cfg, const double* line,
                          int line_per_stream, void* stream);
 
-/* One whole tick in one call: dd_tracker_predict + dd_tracker_update + dd_tracker_countline and, when
- * out_counts != NULL, dd_tracker_count_reduce (7 kernel launches on `stream`). */
-int dd_tracker_tick(void* state, const dd_tracker_config* host_cfg, const double* det_tlwh,
-                    const float* det_conf, const int32_t* det_label, const float* det_feat,
-                    const int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                    int line_per_stream, int64_t* out_counts, void* stream);
-
-/* dd_tracker_tick that also records eight caller-supplied CUDA events on `stream` (before the first kernel and after
- * each of prep / gate / gallery / match / apply / count-line / count-reduce), so that a benchmark can draw the kernel
- * timeline of several stream chunks running concurrently.  host_events8: host array of dd_event_create events. */
-int dd_tracker_tick_profiled(void* state, const dd_tracker_config* host_cfg, const double* det_tlwh,
-                             const float* det_conf, const int32_t* det_label, const float* det_feat,
-                             const int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                             int line_per_stream, int64_t* out_counts, void* stream, void* const* host_events8);
-
-/* Ragged detection batch -> the padded arrays dd_tracker_tick consumes.  The reference hands Tracker.update a
+/* Ragged detection batch -> the padded arrays dd_tracker_update consumes.  The reference hands Tracker.update a
  * Python list of Detection objects per stream (deepdish.py:1014); its batched equivalent is one contiguous blob
  * (what a host uploads with a single copy):  i32 offsets[S+1] (stream s owns entries offsets[s]..offsets[s+1]),
  * then at the given byte offsets f64 tlwh[N][4], f32 conf[N], i32 label[N], f32 feat[N][128], N = offsets[S].
@@ -251,15 +229,6 @@ int dd_tracker_tick_profiled(void* state, const dd_tracker_config* host_cfg, con
 int dd_unpack_detections(const void* blob, int32_t n_streams, int32_t max_dets, int64_t off_tlwh, int64_t off_conf,
                          int64_t off_label, int64_t off_feat, double* det_tlwh, float* det_conf,
                          int32_t* det_label, float* det_feat, int32_t* det_count, void* stream);
-
-/* dd_tracker_tick fed directly by a ragged blob (the format of dd_unpack_detections): the first kernel of the tick
- * expands box / confidence / label / count into the caller's padded arrays det_tlwh f64 [S,Dmax,4], det_conf f32 [S,Dmax],
- * det_label i32 [S,Dmax], det_count i32 [S] (read by the later kernels) and normalises the features straight from the
- * blob -- no padded copy of the 512-byte feature rows. */
-int dd_tracker_tick_ragged(void* state, const dd_tracker_config* host_cfg, const void* blob, int64_t off_tlwh,
-                           int64_t off_conf, int64_t off_label, int64_t off_feat, double* det_tlwh, float* det_conf,
-                           int32_t* det_label, int32_t* det_count, int32_t* out_det_track_id, const double* line,
-                           int line_per_stream, int64_t* out_counts, void* stream);
 
 /* Sum the per-stream counters into out_counts i64 [C,4] (the tensor handed to the NCCL all-reduce). */
 int dd_tracker_count_reduce(void* state, const dd_tracker_config* host_cfg, int64_t* out_counts,
@@ -274,7 +243,7 @@ int dd_tracker_status(void* state, const dd_tracker_config* host_cfg, int32_t* h
  * deepdish.py:1245-1262 -> Pipeline.process_results :1035-1114 around Tracker.predict / update).  One engine drives
  * the n_chunks trackers ("stream chunks": contiguous blocks of streams with their own state blob and CUDA stream) of
  * one GPU: per chunk and tick the detection-prep kernel launched with the tick's inputs by value -- it publishes them into the
- * blob's tick_args words -- followed by ONE captured CUDA graph of the remaining 6-7 kernels of dd_tracker_tick; chunks overlap freely across tick
+ * blob's tick_args words -- followed by ONE captured CUDA graph of the remaining kernels of the tick; chunks overlap freely across tick
  * boundaries; the chunks' partial counters are summed into total_counts on the auxiliary stream.
  * The engine is a HOST object owning only CUDA events / graphs / one capture stream / per-chunk copy streams and 32
  * bytes of pinned memory per chunk; all device buffers stay caller-owned.  Not thread-safe.

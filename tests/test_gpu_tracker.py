@@ -12,7 +12,8 @@ from tests.parity import OracleStreams, compare_stream, compare_costs, LABELS3
 pytestmark = pytest.mark.gpu
 
 
-def _run(S, nobj, dmax, tmax, frames, max_age, seed, budget=100, check_every=1, **kw):
+def _run(S, nobj, dmax, tmax, frames, max_age, seed, budget=100, check_every=1, per_call=False, **kw):
+    """per_call: every tick issued call by call (predict, update, countline) instead of through the engine."""
     from deepdish_b200.batched import BatchedTracker
     bt = BatchedTracker(S, LABELS3, max_tracks=tmax, max_dets=dmax, budget=budget, max_age=max_age, **kw)
     orc = OracleStreams(S, LABELS3, budget=budget, max_age=max_age)
@@ -20,7 +21,13 @@ def _run(S, nobj, dmax, tmax, frames, max_age, seed, budget=100, check_every=1, 
     for f in range(frames):
         b = sc.step()
         ids = orc.step(b)
-        got = bt.step(b.to("cuda")).cpu().numpy()
+        d = b.to("cuda")
+        if per_call:
+            bt.predict()
+            got = bt.update(d.tlwh, d.conf, d.label, d.feat, d.count).cpu().numpy()
+            bt.countline()
+        else:
+            got = bt.step(d).cpu().numpy()
         for s in range(S):
             n = int(b.count[s])
             assert list(got[s, :n]) == ids[s], (f, s)
@@ -62,11 +69,14 @@ def test_small_budget_and_short_age():
 
 def test_unbounded_galleries_and_pool_growth_multi_stream():
     """nn_budget=None on several streams and two chunks, starting from a pool and page tables that are far too small:
-    pool segments are attached and the page tables re-laid out while the run goes on; parity with the oracle throughout."""
-    bt, orc = _run(6, 10, 14, 40, 260, 20, seed=21, budget=None, check_every=13, n_chunks=2,
-                   pool_pages=64, seg_pages=64, page_cap=2)
-    assert all(len(c.segs) > 1 for c in bt.chunks) and all(c.v["ptab"].shape[2] >= 16 for c in bt.chunks)
-    assert max(len(g) for t in orc.trk for g in t.metric.samples.values()) > 200
+    pool segments are attached and the page tables re-laid out while the run goes on -- between engine ticks from the
+    engine's pool polls, and in a second run by update() from the exact counters --; parity with the oracle
+    throughout."""
+    for per_call in (False, True):
+        bt, orc = _run(6, 10, 14, 40, 260, 20, seed=21, budget=None, check_every=13, n_chunks=2,
+                       pool_pages=64, seg_pages=64, page_cap=2, per_call=per_call)
+        assert all(len(c.segs) > 1 for c in bt.chunks) and all(c.v["ptab"].shape[2] >= 16 for c in bt.chunks), per_call
+        assert max(len(g) for t in orc.trk for g in t.metric.samples.values()) > 200
 
 
 def test_pool_exhaustion_is_reported_not_silent():
@@ -139,8 +149,9 @@ def test_gated_cost_matrices_match_oracle():
     assert checked > 1000
 
 
-def test_stream_chunks_pipelined_and_step_host():
-    """n_chunks > 1 (chunk streams, enqueue-only steps, pinned-host entry) gives the same ids / state /
+def test_stream_chunks_engine_host_and_per_call_ticks():
+    """n_chunks > 1, switching tick by tick between the engine on device batches (enqueue-only steps), the engine on
+    ragged pinned host batches and the per-call path (predict, update, countline, reduce_counts): the same ids / state /
     counters as the oracle, and the chunked count reduction equals the sum over streams."""
     from deepdish_b200.batched import BatchedTracker
     S = 7
@@ -161,10 +172,11 @@ def test_stream_chunks_pipelined_and_step_host():
             torch.cuda.synchronize()
             got = ids_host.numpy().copy()
         else:
-            bt.step_host(b.pin(), ids_host)
-            bt.join()
-            torch.cuda.synchronize()
-            got = ids_host.numpy().copy()
+            d = b.to("cuda")
+            bt.predict()
+            got = bt.update(d.tlwh, d.conf, d.label, d.feat, d.count).cpu().numpy()
+            bt.countline()
+            bt.reduce_counts()
         for s in range(S):
             n = int(b.count[s])
             assert list(got[s, :n]) == ids[s], (f, s)
