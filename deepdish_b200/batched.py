@@ -296,6 +296,7 @@ class BatchedTracker:
             if grown:
                 self._rebind(c)
                 c.eng_poll_seen = -1
+                self._after_caller(c)
 
     def memory_bytes(self):
         """Device bytes of the tracker state: blobs + gallery page pool."""
@@ -307,6 +308,15 @@ class BatchedTracker:
     def _sp(self, c):
         s = c.stream if c.stream is not None else self._cur()
         return ctypes.c_void_p(s.cuda_stream)
+
+    def _after_caller(self, c):
+        """Chunk c's stream waits for what the caller's stream holds now: a state edit made there (a re-laid-out blob
+        filled by copies, new pool segments taken from the caller's stream's allocations, a gallery insert).
+        dd_engine_step_host does not fork from the caller's stream, so without this a host-path tick could read the
+        state before the edit.  The blob and the segments are only freed after a host synchronisation of the chunk's
+        stream (re-layout, load_state_dict, the tracker's end), so using them on it needs no record_stream."""
+        if c.stream is not None:
+            c.stream.wait_stream(self._cur())
 
     def _fork(self, tensors=()):
         """Chunk streams wait for everything already enqueued on the caller's stream."""
@@ -470,7 +480,9 @@ class BatchedTracker:
         (dd_engine_step_host).  Per chunk: ONE H2D copy on the chunk's own copy stream into a double-buffered device
         blob -- so the upload of tick k + 1 runs under the kernels of tick k --, then on the chunk's compute stream the
         captured tick reading the blob in place, its partial count reduction and (optionally) the D2H copy of the
-        det->track ids.  The pinned blobs must stay alive until their copy has run.  Returns total_counts (device;
+        det->track ids.  The pinned blobs must stay alive until their copy has run.  Unlike step(), the chunk streams do
+        not wait for the caller's stream; this tracker's own edits made there (maintain(), gallery_insert) are ordered
+        before the next tick of the chunk they touch.  Returns total_counts (device;
         valid on the caller's stream after join() or all_reduce_counts())."""
         self._enter("eng")
         if self._poll_pool:
@@ -665,6 +677,7 @@ class BatchedTracker:
         _lib.check(self.lib.dd_tracker_gallery_insert(c.state, c.cfgp, stream - c.lo, slot, f.data_ptr(),
                                                       1 if before_newest else 0,
                                                       ctypes.c_void_p(self._cur().cuda_stream)), "dd_tracker_gallery_insert")
+        self._after_caller(c)
         if self._poll_pool:
             self.maintain(wait=True)
 

@@ -470,17 +470,23 @@ int dd_engine_pool_latest(void* engine, int32_t chunk, int32_t max_age_ticks, in
     *host_out_tick = -1;
     const int newest = c.poll_turn ^ 1, older = c.poll_turn;          // poll_turn = the slot the NEXT poll writes
     int use = -1;
-    if (c.poll_tick[newest] >= 0) {
-        const cudaError_t q = cudaEventQuery(c.poll_ev[newest]);
-        if (q == cudaSuccess) use = newest;
+    for (const int k : {newest, older}) {                             // the most recent poll that has completed
+        if (use >= 0 || c.poll_tick[k] < 0) continue;
+        const cudaError_t q = cudaEventQuery(c.poll_ev[k]);
+        if (q == cudaSuccess) use = k;
         else if (q != cudaErrorNotReady) return DD_ERR_CUDA;
-        else if (E->tick - c.poll_tick[newest] >= max_age_ticks) {   // the host is too far ahead: wait for it
-            DD_CU(blocked_sync(*E, c.poll_ev[newest]));
-            use = newest;
+    }
+    cudaGetLastError();
+    if (use < 0) {
+        // none has: the host is too far ahead if one of them is max_age_ticks old -- wait for the most recent such poll.
+        // (Waiting only for the newest would never happen once polls come more often than max_age_ticks: a newer poll
+        // always replaces it before it gets that old, and a device that lags a few ticks would never be polled.)
+        for (const int k : {newest, older}) {
+            if (use >= 0 || c.poll_tick[k] < 0 || E->tick - c.poll_tick[k] < max_age_ticks) continue;
+            DD_CU(blocked_sync(*E, c.poll_ev[k]));
+            use = k;
         }
     }
-    if (use < 0 && c.poll_tick[older] >= 0 && cudaEventQuery(c.poll_ev[older]) == cudaSuccess) use = older;
-    cudaGetLastError();
     if (use < 0) return DD_OK;
     for (int k = 0; k < 4; ++k) host_out4[k] = c.poll_host[4 * use + k];
     *host_out_tick = c.poll_tick[use];

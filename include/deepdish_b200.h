@@ -286,7 +286,10 @@ int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, 
  * = byte offsets of chunk i's tlwh / conf / label / feat sections): upload on the chunk's copy stream (the upload of
  * tick k + 1 runs under the kernels of tick k), the tick reading the blob in place, the count reduction, and -- when
  * host_out_ids (pinned, i32 [S,Dmax]) is given -- the device-to-host copy of the det -> track ids.  The host blobs
- * must stay untouched until their copy has run. */
+ * must stay untouched until their copy has run.  With n_chunks > 1 the chunk streams do NOT wait for caller_stream,
+ * so a tick is not held up by whatever the caller queued there: a host that edits a chunk's state or pool on
+ * another stream (re-layout, pool segments, gallery insert) makes the chunk's stream wait for that edit itself, as
+ * BatchedTracker does. */
 int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
                         const int64_t* host_offsets4, int32_t* host_out_ids, void* caller_stream);
 /* caller_stream waits for every chunk and for the latest count summation (no host synchronisation). */
@@ -294,8 +297,9 @@ int dd_engine_join(void* engine, void* caller_stream);
 /* caller_stream waits for the latest count summation only (total_counts of the last reduced tick). */
 int dd_engine_wait_counts(void* engine, void* caller_stream);
 /* Latest completed poll of chunk's pool counters -> host_out4 (free pages, pages attached, longest gallery, forecast)
- * and the tick it was taken behind (-1: none yet).  If the newest poll is still in flight and the engine is already
- * max_age_ticks ticks past it, waits for it: the host never runs further ahead than the forecast covers. */
+ * and the tick it was taken behind (-1: none yet).  If neither of the two most recent polls has completed and the
+ * engine is already max_age_ticks ticks past one of them, waits for the more recent such poll: the host never runs
+ * further ahead than the forecast covers. */
 int dd_engine_pool_latest(void* engine, int32_t chunk, int32_t max_age_ticks, int32_t* host_out4, int64_t* host_out_tick);
 /* Ticks stepped, kernels launched (prep kernels + graph nodes + count summations), host milliseconds spent blocked in the run-ahead
  * throttle.  Any output may be NULL. */

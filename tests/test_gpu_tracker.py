@@ -276,17 +276,18 @@ def test_checkpoint_resume_is_bit_identical():
     assert torch.equal(a.reduce_counts(), b2.reduce_counts())
 
 
+@pytest.mark.parametrize("match_warps", [4, 8])
 @pytest.mark.parametrize("shape", ["crowd", "c3", "small_budget"])
-def test_four_warp_matching_kernel(shape):
-    """k_match_cta (4 warps per stream, picked automatically for crowded scenes) forced on for several shapes: the
-    same oracle parity as the one-warp kernel."""
+def test_cta_matching_kernel(shape, match_warps):
+    """k_match_cta (4 warps per stream, picked automatically for crowded scenes; 8 on request) forced on for several
+    shapes: the same oracle parity as the one-warp kernel."""
     if shape == "crowd":
-        bt, orc = _run(3, 190, 224, 384, 40, 60, seed=18, check_every=5, match_warps=4)
+        bt, orc = _run(3, 190, 224, 384, 40, 60, seed=18, check_every=5, match_warps=match_warps)
         assert max(len(t.tracks) for t in orc.trk) > 200
     elif shape == "c3":
-        _run(12, 50, 64, 128, 70, 60, seed=6, check_every=10, match_warps=4)
+        _run(12, 50, 64, 128, 70, 60, seed=6, check_every=10, match_warps=match_warps)
     else:
-        _run(4, 12, 16, 48, 100, 3, seed=10, budget=5, check_every=4, match_warps=4)
+        _run(4, 12, 16, 48, 100, 3, seed=10, budget=5, check_every=4, match_warps=match_warps)
 
 
 def test_unpack_detections_entry():
