@@ -35,7 +35,8 @@ class TrackerConfig(ctypes.Structure):
 LAYOUT_FIELDS = ["n_tracks", "next_id", "n_deleted", "err", "order", "deleted", "counts", "mean", "cov",
                  "track_id", "hits", "age", "tsu", "state", "gal_len", "gal_pos", "gal_np", "ptab", "free_stack",
                  "pool_ctl", "lab_cnt", "lab_sum", "path_n", "path_last", "path_crossed", "gate", "cost", "det_xyah",
-                 "det_featn", "det_slot", "det_kind", "cdesc", "work", "work_ctl", "work_rec", "det_feath", "tick_args", "timeline"]
+                 "det_featn", "det_slot", "det_kind", "cdesc", "work", "work_ctl", "work_rec", "det_feath", "tick_args", "timeline",
+                 "tick_present"]
 
 
 class TrackerLayout(ctypes.Structure):
@@ -61,6 +62,7 @@ def field_specs(cfg):
         "det_slot": (i, (S, D)), "det_kind": (i, (S, D)), "cdesc": (i, (S, T, 4)),
         "work": (i, (S * T,)), "work_ctl": (i, (64,)), "work_rec": (i, (S * T, 16)),
         "det_feath": ("float16", (S, D, 128)), "tick_args": (i, (64,)), "timeline": ("int64", (64, 8, 2)),
+        "tick_present": (i, (S,)),
     }
 
 
@@ -141,6 +143,9 @@ def lib():
         "dd_engine_bind_host": [_vp, _i32, ctypes.POINTER(_vp), _i32, _u64, _vp, _vp, _vp, _vp],
         "dd_engine_step": [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp],
         "dd_engine_step_host": [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_int64), _vp, _vp],
+        "dd_engine_step_present": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp],
+        "dd_engine_step_host_present": [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_int64), _vp,
+                                        _vp],
         "dd_engine_join": [_vp, _vp],
         "dd_engine_wait_counts": [_vp, _vp],
         "dd_engine_pool_latest": [_vp, _i32, _i32, ctypes.POINTER(_i32), ctypes.POINTER(ctypes.c_int64)],

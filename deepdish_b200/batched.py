@@ -16,6 +16,7 @@ every chunk.  With ``n_chunks=1`` everything runs on the caller's current stream
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -420,22 +421,40 @@ class BatchedTracker:
                                                      self._sp(c)), "dd_tracker_countline")
         self.join()
 
-    def step(self, batch, join=True, reduce=False):
+    def _check_present(self, present):
+        S = self.n_streams
+        if not isinstance(present, torch.Tensor) or present.dtype not in (torch.bool, torch.uint8) \
+                or tuple(present.shape) != (S,) or present.device != self.device or not present.is_contiguous():
+            raise ValueError("present: expected a contiguous bool or uint8 tensor (%d,) on %s, got %s"
+                             % (S, self.device, "%s %s on %s" % (present.dtype, tuple(present.shape), present.device)
+                                if isinstance(present, torch.Tensor) else type(present).__name__))
+
+    def step(self, batch, join=True, reduce=False, present=None):
         """One tick (predict + update + count-line [+ count reduction into total_counts]) for a SceneBatch-like object
         of device tensors: ONE call into the native engine, which launches one captured graph per chunk.  join=False
-        only enqueues (call join())."""
+        only enqueues (call join()).
+
+        present: frame presence of each stream this tick, a contiguous CUDA bool / uint8 tensor [S] on the tracker's
+        device (None: every stream has a frame).  A stream without a frame is left exactly as it is -- no predict, no
+        update, no gallery append, no count-line step, as the reference leaves the tracker of a camera that delivers no
+        frame --, its rows of the batch (count included) are ignored and its det_track_id row is -1.  Its tracks
+        survive any length of absence and are predicted once at its next frame."""
         tlwh, conf, label, feat, count = batch.tlwh, batch.conf, batch.label, batch.feat, batch.count
         self._check_batch(tlwh, conf, label, feat, count)
+        if present is not None:
+            self._check_present(present)
         self._enter("eng")
         if self._poll_pool:
             self.maintain()
         if len(self.chunks) > 1:
-            for t in (tlwh, conf, label, feat, count):
+            for t in (tlwh, conf, label, feat, count) + ((present,) if present is not None else ()):
                 for c in self.chunks:
                     t.record_stream(c.stream)
-        _lib.check(self.lib.dd_engine_step(self._eng(), tlwh.data_ptr(), conf.data_ptr(), label.data_ptr(), feat.data_ptr(),
-                                           count.data_ptr(), 1 if reduce else 0, ctypes.c_void_p(self._cur().cuda_stream)),
-                   "dd_engine_step")
+        _lib.check(self.lib.dd_engine_step_present(self._eng(), tlwh.data_ptr(), conf.data_ptr(), label.data_ptr(),
+                                                   feat.data_ptr(), count.data_ptr(),
+                                                   present.data_ptr() if present is not None else None,
+                                                   1 if reduce else 0, ctypes.c_void_p(self._cur().cuda_stream)),
+                   "dd_engine_step_present")
         self._tick += 1
         if join:
             self.join()
@@ -451,23 +470,32 @@ class BatchedTracker:
                                torch.empty((n,), dtype=torch.int32, device=self.device))
         return c.staging_small
 
-    def pack_host(self, batch):
+    def pack_host(self, batch, present=None):
         """Ragged host form of a padded batch (the batched equivalent of the reference's per-stream list of
         Detection objects, deepdish.py:1014): per chunk ONE pinned byte blob
         ``[i32 offsets[n+1] | f64 tlwh[N,4] | f32 conf[N] | i32 label[N] | f32 feat[N,128]]`` holding only the
-        detections that exist, so a tick uploads one copy per chunk and no padding."""
+        detections that exist, so a tick uploads one copy per chunk and no padding.
+        present: frame presence of each stream (bool-like [S], host or device; see step()).  Each blob then ends with
+        a ``u8 present[n]`` section, absent streams own no entries and their counts are ignored; the presence rides in
+        the tick's one upload."""
         from . import ragged
         cnt = batch.count.cpu().numpy()
         tlwh, conf = batch.tlwh.cpu().numpy(), batch.conf.cpu().numpy()
         label, feat = batch.label.cpu().numpy(), batch.feat.cpu().numpy()
+        if present is not None:
+            present = (present.cpu().numpy() if isinstance(present, torch.Tensor) else np.asarray(present)).astype(bool)
+            if present.shape != (self.n_streams,):
+                raise ValueError("present must have shape (%d,), got %s" % (self.n_streams, present.shape))
+            cnt = np.where(present, cnt, 0)
         if int(cnt.max(initial=0)) > self.max_dets:
             raise RuntimeError("detection capacity exceeded (max_dets=%d)" % self.max_dets)
         out = []
         for c in self.chunks:
-            _, total = ragged.section_offsets(c.hi - c.lo, int(cnt[c.lo:c.hi].sum()))
+            pr = present[c.lo:c.hi] if present is not None else None
+            _, total = ragged.section_offsets(c.hi - c.lo, int(cnt[c.lo:c.hi].sum()), pr is not None)
             blob = torch.empty(max(total, 16), dtype=torch.uint8).pin_memory()
             _, total, sections = ragged.pack(tlwh[c.lo:c.hi], conf[c.lo:c.hi], label[c.lo:c.hi], feat[c.lo:c.hi],
-                                             cnt[c.lo:c.hi], out=blob.numpy())
+                                             cnt[c.lo:c.hi], out=blob.numpy(), present=pr)
             out.append((blob, total, sections))
         return out
 
@@ -483,7 +511,14 @@ class BatchedTracker:
         det->track ids.  The pinned blobs must stay alive until their copy has run.  Unlike step(), the chunk streams do
         not wait for the caller's stream; this tracker's own edits made there (maintain(), gallery_insert) are ordered
         before the next tick of the chunk they touch.  Returns total_counts (device;
-        valid on the caller's stream after join() or all_reduce_counts())."""
+        valid on the caller's stream after join() or all_reduce_counts()).
+        A batch packed with frame presence (``pack_host(batch, present)``) runs the tick of step(present=...)
+        (dd_engine_step_host_present); every chunk of it must carry the presence section or none."""
+        kinds = {len(p[2]) for p in packed}
+        if len(packed) != len(self.chunks) or not kinds <= {4, 5} or len(kinds) != 1:
+            raise ValueError("packed: expected one blob per chunk (%d), all with or all without a presence section"
+                             % len(self.chunks))
+        n_off = kinds.pop()
         self._enter("eng")
         if self._poll_pool:
             self.maintain()
@@ -492,21 +527,21 @@ class BatchedTracker:
         if getattr(self, "_host_bound", None) is None:
             for i, c in enumerate(self.chunks):
                 n = c.hi - c.lo
-                cap = 4 * (n + 1) + 64 + n * self.max_dets * (32 + 4 + 4 + 512)
+                cap = 4 * (n + 1) + 64 + n * self.max_dets * (32 + 4 + 4 + 512) + n + 16
                 c.blob_dev = [torch.empty(cap, dtype=torch.uint8, device=self.device) for _ in range(self.UPLOAD_BUFFERS)]
                 ptrs = (ctypes.c_void_p * len(c.blob_dev))(*[b.data_ptr() for b in c.blob_dev])
                 t, cf, lb, ct = self._staging_small(c)
                 _lib.check(self.lib.dd_engine_bind_host(eng, i, ptrs, len(c.blob_dev), cap,
                                                         t.data_ptr(), cf.data_ptr(), lb.data_ptr(), ct.data_ptr()),
                            "dd_engine_bind_host")
-            self._host_bound = ((ctypes.c_void_p * P)(), (ctypes.c_uint64 * P)(), (ctypes.c_int64 * (4 * P))())
+            self._host_bound = ((ctypes.c_void_p * P)(), (ctypes.c_uint64 * P)(), (ctypes.c_int64 * (5 * P))())
         blobs, sizes, offs = self._host_bound
         for i, (blob, total, sec) in enumerate(packed):
             blobs[i], sizes[i] = blob.data_ptr(), total
-            offs[4 * i], offs[4 * i + 1], offs[4 * i + 2], offs[4 * i + 3] = sec
-        _lib.check(self.lib.dd_engine_step_host(eng, blobs, sizes, offs,
-                                                out_ids_host.data_ptr() if out_ids_host is not None else None,
-                                                ctypes.c_void_p(self._cur().cuda_stream)), "dd_engine_step_host")
+            offs[n_off * i:n_off * (i + 1)] = list(sec)
+        fn = self.lib.dd_engine_step_host_present if n_off == 5 else self.lib.dd_engine_step_host
+        _lib.check(fn(eng, blobs, sizes, offs, out_ids_host.data_ptr() if out_ids_host is not None else None,
+                      ctypes.c_void_p(self._cur().cuda_stream)), fn.__name__)
         self._tick += 1
         return self.total_counts
 
@@ -640,7 +675,7 @@ class BatchedTracker:
 
     def host_view(self, names=None, streams=None):
         """numpy copies of state arrays (optionally a subset of streams) for inspection / tests."""
-        names = names or [n for n in self.v.keys() if n not in ("ptab", "free_stack", "pool_ctl", "work_rec", "cost", "gate", "det_featn", "det_feath", "work", "work_ctl", "tick_args", "timeline")]
+        names = names or [n for n in self.v.keys() if n not in ("ptab", "free_stack", "pool_ctl", "work_rec", "cost", "gate", "det_featn", "det_feath", "work", "work_ctl", "tick_args", "timeline", "tick_present")]
         out = {}
         for n in names:
             t = self.v[n]

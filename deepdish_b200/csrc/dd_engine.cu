@@ -333,6 +333,12 @@ int dd_engine_bind_host(void* engine, int32_t chunk, void* const* host_dev_blobs
 
 int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, const int32_t* det_label,
                    const float* det_feat, const int32_t* det_count, int32_t reduce, void* caller_stream) {
+    return dd_engine_step_present(engine, det_tlwh, det_conf, det_label, det_feat, det_count, nullptr, reduce, caller_stream);
+}
+
+int dd_engine_step_present(void* engine, const double* det_tlwh, const float* det_conf, const int32_t* det_label,
+                           const float* det_feat, const int32_t* det_count, const uint8_t* present, int32_t reduce,
+                           void* caller_stream) {
     Engine* E = (Engine*)engine;
     if (!E || !det_tlwh || !det_conf || !det_label || !det_feat || !det_count) return DD_ERR_INVALID;
     cudaStream_t cur = (cudaStream_t)caller_stream;
@@ -354,6 +360,7 @@ int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, 
         A.out_ids = E->ids + o;
         A.out_counts = reduce ? E->partial + ((size_t)par * E->P + i) * E->C4 : nullptr;
         A.blob = nullptr;
+        A.present = present ? present + c.lo : nullptr;
         A.off_tlwh = A.off_conf = A.off_label = A.off_feat = 0;
         A.indirect = 0;
         A.tick = (int)E->tick;
@@ -370,17 +377,22 @@ int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, 
     return DD_OK;
 }
 
-int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
-                        const int64_t* host_offsets4, int32_t* host_out_ids, void* caller_stream) {
-    Engine* E = (Engine*)engine;
-    if (!E || !host_blobs || !host_blob_bytes || !host_offsets4) return DD_ERR_INVALID;
+}  // extern "C"
+
+namespace {
+
+// n_off: offsets per chunk in host_offsets, 4 (tlwh, conf, label, feat) or 5 (+ the u8 present[n] section)
+int step_host(Engine* E, const void* const* host_blobs, const uint64_t* host_blob_bytes, const int64_t* host_offsets,
+              int n_off, int32_t* host_out_ids, void* caller_stream) {
+    if (!E || !host_blobs || !host_blob_bytes || !host_offsets) return DD_ERR_INVALID;
     cudaStream_t cur = (cudaStream_t)caller_stream;
     const int par = (int)(E->tick & 1);
     const bool multi = E->P > 1;
     for (int i = 0; i < E->P; ++i) {
-        const int64_t* of = host_offsets4 + 4 * i;
+        const int64_t* of = host_offsets + n_off * i;
         if (!host_blobs[i] || E->ch[i].n_blob < 2 || host_blob_bytes[i] > E->ch[i].blob_cap) return DD_ERR_INVALID;
         if ((of[0] & 7) || (of[1] & 3) || (of[2] & 3) || (of[3] & 15)) return DD_ERR_INVALID;
+        if (n_off == 5 && (of[4] < 0 || (uint64_t)of[4] + (uint64_t)E->ch[i].n > host_blob_bytes[i])) return DD_ERR_INVALID;
     }
     if (multi && E->sum_valid[par])
         for (auto& c : E->ch) DD_CU(cudaStreamWaitEvent(c.st, E->sum_done[par], 0));
@@ -408,13 +420,14 @@ int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint6
             DD_CU(cudaStreamWaitEvent(st, c.copied2, 0));
         }
         const size_t o = (size_t)c.lo * E->D;
-        const int64_t* of = host_offsets4 + 4 * i;
+        const int64_t* of = host_offsets + n_off * i;
         DDTickArgs A;
         A.det_tlwh = c.s_tlwh; A.det_conf = c.s_conf; A.det_label = c.s_label; A.det_feat = nullptr; A.det_count = c.s_count;
         A.out_ids = E->ids + o;
         A.out_counts = E->partial + ((size_t)par * E->P + i) * E->C4;
         A.blob = c.dev_blob[bi];
         A.off_tlwh = of[0]; A.off_conf = of[1]; A.off_label = of[2]; A.off_feat = of[3];
+        A.present = n_off == 5 ? c.dev_blob[bi] + of[4] : nullptr;     // rides in the same upload
         A.indirect = 0;
         A.tick = (int)E->tick;
         // only the tick's first kernel reads the blob (later kernels read the small padded arrays it fills)
@@ -440,6 +453,20 @@ int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint6
     if (rc != DD_OK) return rc;
     ++E->tick;
     return DD_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
+                        const int64_t* host_offsets4, int32_t* host_out_ids, void* caller_stream) {
+    return step_host((Engine*)engine, host_blobs, host_blob_bytes, host_offsets4, 4, host_out_ids, caller_stream);
+}
+
+int dd_engine_step_host_present(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
+                                const int64_t* host_offsets5, int32_t* host_out_ids, void* caller_stream) {
+    return step_host((Engine*)engine, host_blobs, host_blob_bytes, host_offsets5, 5, host_out_ids, caller_stream);
 }
 
 int dd_engine_join(void* engine, void* caller_stream) {

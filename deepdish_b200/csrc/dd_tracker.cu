@@ -42,7 +42,7 @@ k_prep(const DDView V, const DDTickArgs A) {
     }
     if (w >= V.S * V.D) return;
     SubG<DD_SUB> g;
-    dd_prep_det(g, V, w / V.D, w % V.D, det_tlwh, det_feat, det_count);
+    dd_prep_det(g, V, w / V.D, w % V.D, det_tlwh, det_feat, det_count, DD_ARG(present));
 }
 
 __global__ void __launch_bounds__(DD_WARPS * 32) k_predict(const DDView V) {
@@ -84,6 +84,7 @@ k_prep_ragged(const DDView V, const DDTickArgs A) {
     if (w >= V.S * V.D) return;
     SubG<DD_SUB> g;
     const int s = w / V.D, d = w - s * V.D;
+    if (!dd_prep_presence(g, V, s, d, DD_ARG(present))) return;     // an absent stream owns no entries
     const int* offs = (const int*)R.blob;
     const int o0 = offs[s];
     const int n = offs[s + 1] - o0;
@@ -120,7 +121,7 @@ k_gate(const DDView V, const DDTickArgs A) {
     int has = 0;
     if (w < V.S * V.T) {
         if (PREDICT) {
-            dd_predict_track(g, V, w / V.T, w % V.T);
+            dd_tick_predict_track(g, V, w / V.T, w % V.T);
             g.sync();
         }
         has = dd_gate_track(g, V, w / V.T, w % V.T, det_count) > 0 ? 1 : 0;
@@ -494,7 +495,7 @@ static DDTickArgs dd_args_padded(const double* det_tlwh, const float* det_conf, 
                                  const int* det_count, int* out_ids) {
     DDTickArgs A;
     A.det_tlwh = det_tlwh; A.det_conf = det_conf; A.det_label = det_label; A.det_feat = det_feat; A.det_count = det_count;
-    A.out_ids = out_ids; A.out_counts = nullptr; A.blob = nullptr;
+    A.out_ids = out_ids; A.out_counts = nullptr; A.blob = nullptr; A.present = nullptr;
     A.off_tlwh = A.off_conf = A.off_label = A.off_feat = 0;
     A.indirect = 0;
     A.tick = 0;

@@ -1,6 +1,6 @@
 // dd_tracker_bodies.cuh -- per-unit bodies of the batched DeepSORT tick (group-generic, see dd_common.cuh).
 //
-//   dd_prep_det        (stream, det)    Detection.to_xyah + feature normalisation
+//   dd_prep_det        (stream, det)    frame presence + Detection.to_xyah + feature normalisation
 //   dd_predict_track   (stream, track)  Track.predict
 //   dd_gate_track      (stream, track)  gating_distance -> gate bitmask + stream descriptor
 //   dd_cosine_track    (stream, track)  gallery min cosine distance for the gate-passing pairs
@@ -141,9 +141,21 @@ DD_HD void dd_prep_det_at(const G& g, const DDView& V, int s, int d, const doubl
     }
 }
 
+// Frame presence (present u8 [S], NULL = every stream): the detection prep of every tick records it in tick_present,
+// which every later step of the tick reads.  A stream without a frame is left exactly as it is -- what the reference
+// does to the tracker of a camera that delivers no frame: no predict, no update, no count-line step -- and its
+// detection inputs are never used.  Returns whether stream s is present.
+template <class G>
+DD_HD bool dd_prep_presence(const G& g, const DDView& V, int s, int d, const unsigned char* present) {
+    const bool p = present == nullptr || present[s] != 0;
+    if (d == 0 && g.lane == 0) V.tick_present[s] = p ? 1 : 0;
+    return p;
+}
+
 template <class G>
 DD_HD void dd_prep_det(const G& g, const DDView& V, int s, int d, const double* det_tlwh,
-                       const float* det_feat, const int* det_count) {
+                       const float* det_feat, const int* det_count, const unsigned char* present = nullptr) {
+    if (!dd_prep_presence(g, V, s, d, present)) return;
     int nd = det_count[s];
     if (nd > V.D) nd = V.D;
     if (d >= nd) return;
@@ -155,14 +167,25 @@ DD_HD void dd_prep_det(const G& g, const DDView& V, int s, int d, const double* 
 // Track.predict (deep_sort/track.py:113-125).
 // ------------------------------------------------------------------------------------------------
 template <class G>
-DD_HD void dd_predict_track(const G& g, const DDView& V, int s, int t) {
-    if (t >= V.n_tracks[s]) return;
+DD_HD void dd_predict_live_track(const G& g, const DDView& V, int s, int t) {
     const size_t slot = (size_t)s * V.T + V.order[(size_t)s * V.T + t];
     dd_kf_predict(g, V.mean + slot * 8, V.cov + slot * 64);
     if (g.lane == 0) {
         V.age[slot] += 1;
         V.tsu[slot] += 1;
     }
+}
+template <class G>
+DD_HD void dd_predict_track(const G& g, const DDView& V, int s, int t) {
+    if (t < V.n_tracks[s]) dd_predict_live_track(g, V, s, t);
+}
+
+// Track.predict inside a tick: only the tracks of a stream that has a frame (the per-call predict steps every stream).
+// The presence word is loaded beside the track count, not in front of it: no extra memory round trip on the chain.
+template <class G>
+DD_HD void dd_tick_predict_track(const G& g, const DDView& V, int s, int t) {
+    const int nt = V.n_tracks[s], present = V.tick_present[s];
+    if (present && t < nt) dd_predict_live_track(g, V, s, t);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -279,10 +302,12 @@ struct DDDirectPass {
 
 // Gate of one track index (every t < Tmax is visited so that inactive entries get an empty descriptor):
 // f64 projection + 4x4 Cholesky per lane (redundant), lanes sweep the detections, ballot -> gate words.
+// A stream without a frame this tick gets empty descriptors only: nothing of it reaches the gallery kernel.
 template <class G>
 DD_HD int dd_gate_track(const G& g, const DDView& V, int s, int t, const int* det_count) {
     int* desc = V.cdesc + ((size_t)s * V.T + t) * 4;
-    bool active = t < V.n_tracks[s];
+    const int nt = V.n_tracks[s], present = V.tick_present[s];
+    bool active = present != 0 && t < nt;
     size_t slot = 0;
     if (active) {
         slot = (size_t)s * V.T + V.order[(size_t)s * V.T + t];
@@ -550,18 +575,21 @@ DD_HD void dd_match_stream(const G& g, const DDView& V, int s, const double* det
     DDMatchSmem m;
     dd_match_carve(smem, V.T, V.D, V.tab_cap, m);
     const size_t sT = (size_t)s * V.T, sD = (size_t)s * V.D;
+    // the count is loaded beside the presence word, off the warp's dependency chain; it is used only when present
+    const int present = V.tick_present[s], nT = V.n_tracks[s], ndel_prev = V.n_deleted[s];
     int nd = det_count[s];
+    if (!present) {                    // no frame: no detections to report, every track and slot stays as it is
+        if (out_det_track_id)
+            for (int d = g.lane; d < V.D; d += G::NL) out_det_track_id[sD + d] = -1;
+        return;
+    }
     if (nd > V.D) {
         nd = V.D;
         if (g.lane == 0) V.err[s] |= DD_FLAG_DET_OVERFLOW;
     }
     if (nd < 0) nd = 0;
-    const int nT = V.n_tracks[s];
     // slots deleted by the previous update become free now
-    {
-        const int ndel = V.n_deleted[s];
-        for (int k = g.lane; k < ndel; k += G::NL) V.state[sT + V.deleted[sT + k]] = DD_STATE_FREE;
-    }
+    for (int k = g.lane; k < ndel_prev; k += G::NL) V.state[sT + V.deleted[sT + k]] = DD_STATE_FREE;
     // Staging loops of this function: the compiler cannot move a global load over the shared-memory store of the
     // iteration before it, so a plain loop pays one memory round trip per iteration -- and this warp is all latency.
     // They are therefore written in batches of DD_MB iterations: all loads of a batch first, then its stores.
@@ -905,8 +933,9 @@ template <class G>
 DD_HD void dd_apply_det(const G& g, const DDView& V, int s, int d, const float* det_conf,
                         const int* det_label, double* scratch) {
     const size_t sd = (size_t)s * V.D + d;
-    const int kind = V.det_kind[sd];
-    if (kind == 0) return;
+    // det_kind of a stream without a frame still holds what its last present tick matched
+    const int present = V.tick_present[s], kind = V.det_kind[sd];
+    if (!present || kind == 0) return;
     const size_t slot = (size_t)s * V.T + V.det_slot[sd];
     const double* z = V.det_xyah + sd * 4;
     // everything the tail needs is loaded before the Kalman arithmetic (independent of it; the compiler cannot
@@ -1024,8 +1053,11 @@ DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) 
     const size_t sT = (size_t)s * V.T;
     const double p1x = line[0], p1y = line[1], q1x = line[2], q1y = line[3];
     long long* cnt = V.counts + (size_t)s * V.C * 4;
+    const int present = V.tick_present[s], ndel = V.n_deleted[s], nT = V.n_tracks[s];
+    // a stream without a frame in the last tick takes no count-line step: in particular the last track its previous
+    // present tick deleted is not counted a second time
+    if (!present) return;
     // deleted tracks (deepdish.py:1041-1044): only the LAST one's result survives the overwrite
-    const int ndel = V.n_deleted[s];
     if (g.lane == 0 && ndel > 0) {
         const size_t slot = sT + V.deleted[sT + ndel - 1];
         if (V.path_n[slot] > 1 && V.path_crossed[slot]) {
@@ -1033,7 +1065,6 @@ DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) 
             if (l >= 0) dd_atomic_add_ll(cnt + l * 4 + 3, 1);
         }
     }
-    const int nT = V.n_tracks[s];
     for (int t = g.lane; t < nT; t += G::NL) {
         const size_t slot = sT + V.order[sT + t];
         if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) continue;

@@ -16,6 +16,8 @@ struct DDTickArgs {
     int* out_ids;                // i32 [S,D] or NULL
     long long* out_counts;       // i64 [C,4] or NULL
     const unsigned char* blob;   // ragged batch (dd_unpack_detections' format) or NULL
+    const unsigned char* present;// u8 [S]: frame presence of each stream, NULL = every stream present (read by the
+                                 // detection-prep kernel only, which records it in the blob's tick_present words)
     long long off_tlwh, off_conf, off_label, off_feat;
     int indirect;
     int tick;                    // engine tick number (timeline slot)
@@ -62,6 +64,7 @@ struct DDView {
     int *det_slot, *det_kind;
     int* cdesc;
     int *work, *work_ctl, *work_rec;
+    int* tick_present;               // [S] 1: the stream has a frame this tick (see dd_prep_presence)
     unsigned short* det_feath;
     const DDTickArgs* targs;         // the blob's tick_args words
     unsigned long long* tl;          // timeline words, NULL unless config.timeline
@@ -164,6 +167,7 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     DD_PUT(det_feath, 2 * S * D * F);
     DD_PUT(tick_args, 256);
     DD_PUT(timeline, 8 * 64 * 8 * 2);
+    DD_PUT(tick_present, 4 * S);
 #undef DD_PUT
     L->total_bytes = off;
     return DD_OK;
@@ -203,6 +207,7 @@ static inline int dd_make_view(void* blob, const dd_tracker_config* c, DDView* v
     v->det_xyah = (double*)(b + L.det_xyah); v->det_featn = (float*)(b + L.det_featn);
     v->det_slot = (int*)(b + L.det_slot); v->det_kind = (int*)(b + L.det_kind);
     v->cdesc = (int*)(b + L.cdesc);
+    v->tick_present = (int*)(b + L.tick_present);
     v->det_feath = (unsigned short*)(b + L.det_feath);
     v->targs = (const DDTickArgs*)(b + L.tick_args);
     v->tl = c->timeline ? (unsigned long long*)(b + L.timeline) : nullptr;

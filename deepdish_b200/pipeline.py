@@ -105,9 +105,10 @@ class DetectTrackPipeline:
                 self.flags.data_ptr() + fe.lo * 4, st), "dd_gather_detections")
         return self.det_tlwh, self.det_conf, self.det_label, self.det_count
 
-    def step(self, heads, features, join=True):
+    def step(self, heads, features, join=True, present=None):
         """detect() + one tracker tick.  features: f32 [S,Dmax,128] tensor or callable(tlwh, count) -> tensor
-        (the re-ID encoder's output for the kept boxes, in the same order)."""
+        (the re-ID encoder's output for the kept boxes, in the same order).  present: frame presence of each stream
+        (BatchedTracker.step): the tick leaves the streams without a frame untouched."""
         tlwh, conf, label, count = self.detect(heads)
         feat = features(tlwh, count) if callable(features) else features
 
@@ -115,7 +116,7 @@ class DetectTrackPipeline:
             pass
         b = _B()
         b.tlwh, b.conf, b.label, b.feat, b.count = tlwh, conf, label, feat, count
-        return self.bt.step(b, join=join, reduce=True)
+        return self.bt.step(b, join=join, reduce=True, present=present)
 
     def check(self):
         if int(self.flags.max()) & _lib.FLAG_DET_OVERFLOW:

@@ -159,6 +159,8 @@ typedef struct dd_tracker_layout {
     uint64_t timeline;      /* u64 [64,8,2]       config.timeline: per engine tick (mod 64) and kernel (prep, gate, gallery, match,
                                                   apply, count-line, count-reduce): min start / max end in ns; the caller
                                                   initialises starts to ~0 and ends to 0                         */
+    uint64_t tick_present;  /* i32 [S]            1: the stream had a frame in the last tick (written by every tick's
+                                                  detection prep; the per-call update marks every stream present)  */
 } dd_tracker_layout;
 
 /* Host-only arithmetic: fills `host_out`.  No CUDA call. */
@@ -214,7 +216,8 @@ int dd_event_destroy(void* ev);
 int dd_event_elapsed_ms(void* start, void* end, float* host_ms);   /* both events must have completed */
 int dd_event_record(void* ev, void* stream);
 
-/* Count-line step (deepdish.py:1035-1114 counting part, :1303-1312; tools/intersection.py:4-30).
+/* Count-line step (deepdish.py:1035-1114 counting part, :1303-1312; tools/intersection.py:4-30).  Skips a stream
+ * that had no frame in the last tick (tick_present; only dd_engine_step_present / _host_present leave one).
  *   line f64 [S,4] (x1,y1,x2,y2 per stream) or, with line_per_stream = 0, one f64[4] for all streams. */
 int dd_tracker_countline(void* state, const dd_tracker_config* host_cfg, const double* line,
                          int line_per_stream, void* stream);
@@ -282,6 +285,15 @@ int dd_engine_bind_host(void* engine, int32_t chunk, void* const* host_dev_blobs
  * enqueues: chunk streams wait for what is already on caller_stream, nothing waits for the chunks. */
 int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, const int32_t* det_label,
                    const float* det_feat, const int32_t* det_count, int32_t reduce, void* caller_stream);
+/* dd_engine_step for a tick in which only some streams have a frame (cameras at different frame rates, dropped
+ * frames): present u8 [S] (nonzero = the stream has a frame; NULL = every stream, which is dd_engine_step).  A stream
+ * without a frame is left exactly as it is, as the reference leaves the Tracker of a camera that delivers no frame:
+ * no Track.predict, no matching or lifecycle change, no gallery append, no count-line step; its rows of the detection
+ * arrays and its det_count are ignored (never used) and its det_track_id row is set to -1.  Its counters still take part in the
+ * count reduction.  Tracks survive any length of absence and are predicted once at the stream's next frame. */
+int dd_engine_step_present(void* engine, const double* det_tlwh, const float* det_conf, const int32_t* det_label,
+                           const float* det_feat, const int32_t* det_count, const uint8_t* present, int32_t reduce,
+                           void* caller_stream);
 /* One end-to-end tick from ragged PINNED host blobs (one per chunk, dd_unpack_detections' format; host_offsets4[4 i ..]
  * = byte offsets of chunk i's tlwh / conf / label / feat sections): upload on the chunk's copy stream (the upload of
  * tick k + 1 runs under the kernels of tick k), the tick reading the blob in place, the count reduction, and -- when
@@ -292,6 +304,11 @@ int dd_engine_step(void* engine, const double* det_tlwh, const float* det_conf, 
  * BatchedTracker does. */
 int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
                         const int64_t* host_offsets4, int32_t* host_out_ids, void* caller_stream);
+/* dd_engine_step_host with frame presence (semantics as dd_engine_step_present): host_offsets5[5 i ..] = chunk i's
+ * tlwh / conf / label / feat offsets and the byte offset of a u8 present[n] section (n = the chunk's streams) inside
+ * its blob, which must lie within host_blob_bytes[i].  An absent stream owns no entries of the blob. */
+int dd_engine_step_host_present(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
+                                const int64_t* host_offsets5, int32_t* host_out_ids, void* caller_stream);
 /* caller_stream waits for every chunk and for the latest count summation (no host synchronisation). */
 int dd_engine_join(void* engine, void* caller_stream);
 /* caller_stream waits for the latest count summation only (total_counts of the last reduced tick). */
