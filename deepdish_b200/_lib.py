@@ -28,7 +28,7 @@ class TrackerConfig(ctypes.Structure):
                 ("label_rank", _i32 * DD_MAX_LABELS),
                 ("page_cap", _i32), ("seg_pages", _i32), ("n_segs", _i32),
                 ("gallery_impl", _i32), ("cosine_ctas_per_sm", _i32), ("match_warps", _i32),
-                ("gallery_stages", _i32), ("gallery_waves", _i32), ("reserved0", _i32), ("timeline", _i32),
+                ("gallery_stages", _i32), ("gallery_waves", _i32), ("event_cap", _i32), ("timeline", _i32),
                 ("pool_f32", _u64 * DD_MAX_SEGS), ("pool_f16", _u64 * DD_MAX_SEGS)]
 
 
@@ -37,10 +37,12 @@ LAYOUT_FIELDS = ["n_tracks", "next_id", "n_deleted", "err", "order", "deleted", 
                  "pool_ctl", "lab_cnt", "lab_sum", "path_n", "path_last", "path_crossed", "gate", "cost", "det_xyah",
                  "det_featn", "det_slot", "det_kind", "cdesc", "work", "work_ctl", "work_rec", "det_feath", "tick_args", "timeline",
                  "tick_present"]
+# the crossing records: appended after every array above, 0 bytes (offset == total_bytes) unless event_cap > 0
+EVENTS_FIELD = "events"
 
 
 class TrackerLayout(ctypes.Structure):
-    _fields_ = [("total_bytes", _u64)] + [(n, _u64) for n in LAYOUT_FIELDS]
+    _fields_ = [("total_bytes", _u64)] + [(n, _u64) for n in LAYOUT_FIELDS + [EVENTS_FIELD]]
 
 
 def field_specs(cfg):
@@ -63,6 +65,8 @@ def field_specs(cfg):
         "work": (i, (S * T,)), "work_ctl": (i, (64,)), "work_rec": (i, (S * T, 16)),
         "det_feath": ("float16", (S, D, 128)), "tick_args": (i, (64,)), "timeline": ("int64", (64, 8, 2)),
         "tick_present": (i, (S,)),
+        # row 0 = header (records this count-line step produced), rows 1.. = {stream, track_id, label, column}
+        "events": (i, (cfg.event_cap + 1 if cfg.event_cap > 0 else 0, 4)),
     }
 
 
@@ -75,7 +79,7 @@ def page_cap(cfg):
 def make_config(n_streams, max_tracks, max_dets, budget, labels, max_age=30, n_init=3,
                 max_cosine_distance=0.2, max_iou_distance=0.7, page_cap=0, seg_pages=1024,
                 gallery_impl=0, cosine_ctas_per_sm=0, match_warps=0, gallery_stages=0, gallery_waves=0,
-                timeline=0):
+                timeline=0, event_cap=0):
     """Fill a dd_tracker_config from Python values; ``labels`` is the ordered list of label names.
     ``budget=None`` is the reference's nn_budget=None (deepdish.py:515): unbounded galleries (budget 0 in the C
     struct).  The pool segment pointers are filled in by the caller that allocates them."""
@@ -91,7 +95,7 @@ def make_config(n_streams, max_tracks, max_dets, budget, labels, max_age=30, n_i
     cfg.page_cap, cfg.seg_pages, cfg.n_segs = page_cap, seg_pages, 1
     cfg.gallery_impl = GALLERY_IMPLS[gallery_impl] if isinstance(gallery_impl, str) else int(gallery_impl)
     cfg.cosine_ctas_per_sm, cfg.match_warps, cfg.gallery_stages = cosine_ctas_per_sm, match_warps, gallery_stages
-    cfg.gallery_waves, cfg.timeline = gallery_waves, timeline
+    cfg.gallery_waves, cfg.timeline, cfg.event_cap = gallery_waves, timeline, event_cap
     cfg.feat_dim, cfg.n_labels, cfg.max_age, cfg.n_init = 128, len(labels), max_age, n_init
     cfg.max_cosine_distance, cfg.max_iou_distance = max_cosine_distance, max_iou_distance
     cfg.label_motorbike = labels.index("motorbike") if "motorbike" in labels else -1
@@ -146,6 +150,7 @@ def lib():
         "dd_engine_step_present": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp],
         "dd_engine_step_host_present": [_vp, ctypes.POINTER(_vp), ctypes.POINTER(_u64), ctypes.POINTER(ctypes.c_int64), _vp,
                                         _vp],
+        "dd_engine_copy_events": [_vp, _vp, _vp],
         "dd_engine_join": [_vp, _vp],
         "dd_engine_wait_counts": [_vp, _vp],
         "dd_engine_pool_latest": [_vp, _i32, _i32, ctypes.POINTER(_i32), ctypes.POINTER(ctypes.c_int64)],

@@ -14,6 +14,7 @@ matching kernel of one chunk runs under the HBM-bound gallery kernel of another,
 boundaries.  ``step(..., join=False)`` only enqueues; ``join()`` makes the caller's stream wait for
 every chunk.  With ``n_chunks=1`` everything runs on the caller's current stream.
 """
+import collections
 import ctypes
 
 import numpy as np
@@ -23,6 +24,12 @@ from . import _lib
 
 _DT = {"int32": torch.int32, "int64": torch.int64, "float32": torch.float32,
        "float64": torch.float64, "float16": torch.float16}
+
+
+Crossings = collections.namedtuple("Crossings", "stream track_id label column")
+Crossings.__doc__ = """Count-line crossings of one tick, numpy int32 arrays sorted by stream (tracker-wide index) and within a stream
+in the order the reference's ``process_results`` counts them (``tracker.tracks``, then the deleted track): column 0 /
+1 = a live track crossed the line (pos / neg, and int, of ``label``), 3 = the del count of the last deleted track."""
 
 
 def _pow2_at_least(n):
@@ -55,7 +62,7 @@ class _Chunk:
                                     gallery_impl=o.gallery_impl, cosine_ctas_per_sm=o.cosine_ctas_per_sm,
                                     match_warps=o.match_warps, gallery_stages=o.gallery_stages,
                                     gallery_waves=o.gallery_waves,
-                                    timeline=o.timeline)
+                                    timeline=o.timeline, event_cap=o.crossing_capacity)
         self.cfgp = ctypes.byref(self.cfg)
         self.segs = []
         for _ in range(n_segs):
@@ -139,13 +146,19 @@ class BatchedTracker:
                  line=None, frame_size=(640, 480), device="cuda", n_chunks=1,
                  pool_pages=None, pool_fraction=0.5, seg_pages=None, page_cap=0,
                  gallery_impl="default", cosine_ctas_per_sm=0, match_warps=0, gallery_stages=0, gallery_waves=0,
-                 timeline=0, gallery_turns=True, engine_graphs=True):
+                 timeline=0, gallery_turns=True, engine_graphs=True, crossing_capacity=0):
         """budget=None is the reference's nn_budget=None (deepdish.py:515-516): galleries grow without bound; the
         page pool and the per-slot page tables are grown between ticks (``maintain``).
 
         Gallery memory: ``pool_pages`` 16-row pages per chunk (default: ``pool_fraction`` of the worst case
         streams x max_tracks x ceil(budget / 16)), in segments of ``seg_pages``; more segments are attached when
-        fewer than 1/8 of the pages are free.  A pool that still runs dry raises in ``check()``."""
+        fewer than 1/8 of the pages are free.  A pool that still runs dry raises in ``check()``.
+
+        crossing_capacity > 0: every count-line step also lists its crossings (``crossings()``), up to that many
+        records per chunk and tick; 0 (the default) leaves the count-line step exactly as without it."""
+        if int(crossing_capacity) < 0:
+            raise ValueError("crossing_capacity must be >= 0")
+        self.crossing_capacity = int(crossing_capacity)
         self.lib = _lib.lib()
         self.pool_pages, self.pool_fraction, self.seg_pages, self.page_cap = pool_pages, pool_fraction, seg_pages, page_cap
         self.gallery_impl, self.cosine_ctas_per_sm, self.match_warps = gallery_impl, cosine_ctas_per_sm, match_warps
@@ -429,7 +442,7 @@ class BatchedTracker:
                              % (S, self.device, "%s %s on %s" % (present.dtype, tuple(present.shape), present.device)
                                 if isinstance(present, torch.Tensor) else type(present).__name__))
 
-    def step(self, batch, join=True, reduce=False, present=None):
+    def step(self, batch, join=True, reduce=False, present=None, out_events_host=None):
         """One tick (predict + update + count-line [+ count reduction into total_counts]) for a SceneBatch-like object
         of device tensors: ONE call into the native engine, which launches one captured graph per chunk.  join=False
         only enqueues (call join()).
@@ -438,8 +451,14 @@ class BatchedTracker:
         device (None: every stream has a frame).  A stream without a frame is left exactly as it is -- no predict, no
         update, no gallery append, no count-line step, as the reference leaves the tracker of a camera that delivers no
         frame --, its rows of the batch (count included) are ignored and its det_track_id row is -1.  Its tracks
-        survive any length of absence and are predicted once at its next frame."""
+        survive any length of absence and are predicted once at its next frame.
+
+        out_events_host: a buffer of ``new_crossings_buffer()``; the tick's crossing records are copied into it behind
+        the tick (read them with ``crossings(out_events_host)`` once the caller's stream has been synchronised after
+        join())."""
         tlwh, conf, label, feat, count = batch.tlwh, batch.conf, batch.label, batch.feat, batch.count
+        if out_events_host is not None:
+            self._check_crossings_buffer(out_events_host)
         self._check_batch(tlwh, conf, label, feat, count)
         if present is not None:
             self._check_present(present)
@@ -455,6 +474,8 @@ class BatchedTracker:
                                                    present.data_ptr() if present is not None else None,
                                                    1 if reduce else 0, ctypes.c_void_p(self._cur().cuda_stream)),
                    "dd_engine_step_present")
+        if out_events_host is not None:
+            self._copy_events(out_events_host)
         self._tick += 1
         if join:
             self.join()
@@ -503,7 +524,7 @@ class BatchedTracker:
     def packed_nbytes(packed):
         return sum(p[1] for p in packed)
 
-    def step_host_packed(self, packed, out_ids_host=None):
+    def step_host_packed(self, packed, out_ids_host=None, out_events_host=None):
         """End-to-end tick from a ragged pinned host batch (``pack_host``): one call into the native engine
         (dd_engine_step_host).  Per chunk: ONE H2D copy on the chunk's own copy stream into a double-buffered device
         blob -- so the upload of tick k + 1 runs under the kernels of tick k --, then on the chunk's compute stream the
@@ -513,7 +534,10 @@ class BatchedTracker:
         before the next tick of the chunk they touch.  Returns total_counts (device;
         valid on the caller's stream after join() or all_reduce_counts()).
         A batch packed with frame presence (``pack_host(batch, present)``) runs the tick of step(present=...)
-        (dd_engine_step_host_present); every chunk of it must carry the presence section or none."""
+        (dd_engine_step_host_present); every chunk of it must carry the presence section or none.
+        out_events_host: as in step(); the copy runs beside the ids' read-back, off the chunks' compute streams."""
+        if out_events_host is not None:
+            self._check_crossings_buffer(out_events_host)
         kinds = {len(p[2]) for p in packed}
         if len(packed) != len(self.chunks) or not kinds <= {4, 5} or len(kinds) != 1:
             raise ValueError("packed: expected one blob per chunk (%d), all with or all without a presence section"
@@ -542,8 +566,61 @@ class BatchedTracker:
         fn = self.lib.dd_engine_step_host_present if n_off == 5 else self.lib.dd_engine_step_host
         _lib.check(fn(eng, blobs, sizes, offs, out_ids_host.data_ptr() if out_ids_host is not None else None,
                       ctypes.c_void_p(self._cur().cuda_stream)), fn.__name__)
+        if out_events_host is not None:
+            self._copy_events(out_events_host)
         self._tick += 1
         return self.total_counts
+
+    # ------------------------------------------------------------------------------------------
+    def _crossings_words(self):
+        return len(self.chunks) * 4 * (1 + self.crossing_capacity)
+
+    def new_crossings_buffer(self):
+        """Pinned host buffer for ``step(..., out_events_host=)`` / ``step_host_packed(..., out_events_host=)``: every
+        chunk's crossing list (header + ``crossing_capacity`` records)."""
+        if self.crossing_capacity <= 0:
+            raise RuntimeError("crossing records are off: construct the tracker with crossing_capacity > 0")
+        return torch.zeros(self._crossings_words(), dtype=torch.int32).pin_memory()
+
+    def _check_crossings_buffer(self, buf):
+        if self.crossing_capacity <= 0:
+            raise RuntimeError("crossing records are off: construct the tracker with crossing_capacity > 0")
+        if not isinstance(buf, torch.Tensor) or buf.dtype != torch.int32 or buf.is_cuda or not buf.is_pinned() \
+                or not buf.is_contiguous() or buf.numel() != self._crossings_words():
+            raise ValueError("out_events_host: expected a buffer of new_crossings_buffer() (pinned int32 [%d])"
+                             % self._crossings_words())
+
+    def _copy_events(self, buf):
+        _lib.check(self.lib.dd_engine_copy_events(self._eng(), buf.data_ptr(), ctypes.c_void_p(self._cur().cuda_stream)),
+                   "dd_engine_copy_events")
+
+    def crossings(self, host_buffer=None):
+        """The count-line crossings of the last tick (or per-call ``countline()``) as ``Crossings`` arrays.
+        host_buffer: a buffer a step copied them into (valid once that copy has completed: after join() and a
+        synchronisation of the caller's stream); None: read from the device, which joins and synchronises.
+        Raises RuntimeError naming the chunk whose list overflowed crossing_capacity (records are never dropped
+        silently), and when the tracker was built without crossing records."""
+        if self.crossing_capacity <= 0:
+            raise RuntimeError("crossing records are off: construct the tracker with crossing_capacity > 0")
+        cap = self.crossing_capacity
+        if host_buffer is None:
+            self.join()
+            torch.cuda.synchronize(self.device)
+            lists = [c.v["events"].cpu().numpy() for c in self.chunks]
+        else:
+            self._check_crossings_buffer(host_buffer)
+            lists = host_buffer.numpy().reshape(len(self.chunks), cap + 1, 4)
+        parts = []
+        for i, (c, ev) in enumerate(zip(self.chunks, lists)):
+            n = int(ev[0, 0])
+            if n > cap:
+                raise RuntimeError("crossing list of chunk %d (streams %d..%d) overflowed: %d records this tick, "
+                                   "crossing_capacity=%d" % (i, c.lo, c.hi - 1, n, cap))
+            rec = ev[1:1 + n]
+            rec = rec[np.argsort(rec[:, 0], kind="stable")]          # by stream; positions keep the order within one
+            parts.append(rec + np.array([c.lo, 0, 0, 0], dtype=np.int32))
+        r = np.concatenate(parts).astype(np.int32, copy=False)
+        return Crossings(r[:, 0].copy(), r[:, 1].copy(), r[:, 2].copy(), r[:, 3].copy())
 
     def reduce_counts(self):
         """Sum the per-stream counters -> i64 [C,4] (pos, neg, int, del per label), this GPU only.  Runs on the caller's
@@ -675,7 +752,7 @@ class BatchedTracker:
 
     def host_view(self, names=None, streams=None):
         """numpy copies of state arrays (optionally a subset of streams) for inspection / tests."""
-        names = names or [n for n in self.v.keys() if n not in ("ptab", "free_stack", "pool_ctl", "work_rec", "cost", "gate", "det_featn", "det_feath", "work", "work_ctl", "tick_args", "timeline", "tick_present")]
+        names = names or [n for n in self.v.keys() if n not in ("ptab", "free_stack", "pool_ctl", "work_rec", "cost", "gate", "det_featn", "det_feath", "work", "work_ctl", "tick_args", "timeline", "tick_present", "events")]
         out = {}
         for n in names:
             t = self.v[n]

@@ -42,6 +42,7 @@ struct Chunk {
     void* state = nullptr;
     dd_tracker_config cfg;
     int lo = 0, n = 0;
+    size_t events_off = 0;       // byte offset of the blob's `events` section (crossing records)
     cudaStream_t st = nullptr, copy_st = nullptr, copy_st2 = nullptr, d2h_st = nullptr;
     cudaEvent_t done = nullptr, copied = nullptr, copied2 = nullptr, unpacked[4] = {nullptr, nullptr, nullptr, nullptr}, gal_done = nullptr;
     cudaEvent_t tick_end = nullptr, d2h_done = nullptr;      // the det -> track ids leave on their own stream
@@ -248,6 +249,7 @@ int dd_engine_create(int32_t n_chunks, void* const* host_states, const dd_tracke
         c.cfg = *host_cfgs[i];
         c.lo = host_first_stream[i];
         c.n = c.cfg.n_streams;
+        c.events_off = L.events;
         c.st = n_chunks > 1 ? (cudaStream_t)host_streams[i] : nullptr;
         if (i == 0) { E->D = c.cfg.max_dets; E->C4 = c.cfg.n_labels * 4; }
         ok = c.cfg.max_dets == E->D && c.cfg.n_labels * 4 == E->C4 &&
@@ -306,8 +308,10 @@ int dd_engine_rebind(void* engine, int32_t chunk, void* state, const dd_tracker_
     if (!E || chunk < 0 || chunk >= E->P || !state || !host_cfg) return DD_ERR_INVALID;
     Chunk& c = E->ch[chunk];
     drop_graphs(c);                  // the DDView frozen in the captured kernels is stale
+    dd_tracker_layout L;
     c.state = state;
     c.cfg = *host_cfg;
+    c.events_off = dd_layout_compute(host_cfg, &L) == DD_OK ? L.events : 0;     // (an invalid config fails at the next tick)
     c.poll_tick[0] = c.poll_tick[1] = -1;
     return DD_OK;
 }
@@ -467,6 +471,33 @@ int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint6
 int dd_engine_step_host_present(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
                                 const int64_t* host_offsets5, int32_t* host_out_ids, void* caller_stream) {
     return step_host((Engine*)engine, host_blobs, host_blob_bytes, host_offsets5, 5, host_out_ids, caller_stream);
+}
+
+int dd_engine_copy_events(void* engine, int32_t* host_out, void* caller_stream) {
+    Engine* E = (Engine*)engine;
+    if (!E || !host_out) return DD_ERR_INVALID;
+    for (auto& c : E->ch)
+        if (c.cfg.event_cap <= 0) return DD_ERR_INVALID;
+    const bool multi = E->P > 1;
+    size_t o = 0;
+    for (auto& c : E->ch) {
+        const size_t words = 4 + 4 * (size_t)c.cfg.event_cap;
+        const void* src = (const char*)c.state + c.events_off;
+        if (multi) {
+            // off the chunk's stream, as the ids of dd_engine_step_host: the next tick waits for d2h_done
+            if (!c.d2h_st) DD_CU(cudaStreamCreateWithFlags(&c.d2h_st, cudaStreamNonBlocking));
+            DD_CU(cudaEventRecord(c.tick_end, c.st));
+            DD_CU(cudaStreamWaitEvent(c.d2h_st, c.tick_end, 0));
+            DD_CU(cudaMemcpyAsync(host_out + o, src, words * sizeof(int32_t), cudaMemcpyDeviceToHost, c.d2h_st));
+            DD_CU(cudaEventRecord(c.d2h_done, c.d2h_st));
+            c.d2h_valid = true;
+        } else {
+            DD_CU(cudaMemcpyAsync(host_out + o, src, words * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                  (cudaStream_t)caller_stream));
+        }
+        o += words;
+    }
+    return DD_OK;
 }
 
 int dd_engine_join(void* engine, void* caller_stream) {

@@ -6,7 +6,7 @@
 //   gallery kernel persistent grid over the work list     <- the HBM-bound kernel (dd_gallery.cuh)
 //   k_match        stream -> 1 warp (4 / 8 for crowds)    cascade + IoU stage + lifecycle, dynamic shared memory
 //   k_apply        (stream, detection) -> 8 lanes         Kalman update / initiate + gallery append + label vote
-//   k_countline    stream -> 1 warp
+//   k_countline    stream -> 1 warp                       (k_countline_ev: + the crossing records)
 //   k_count_reduce one CTA per counter
 #include <cuda_runtime.h>
 #include "dd_gallery.cuh"
@@ -223,6 +223,17 @@ k_countline(const DDView V, const double* __restrict__ line, int line_per_stream
     dd_countline(g, V, w, line + (line_per_stream ? (size_t)w * 4 : 0));
 }
 
+// k_countline that also writes the crossing records (config.event_cap > 0); a kernel of its own so that k_countline
+// stays exactly what it is when the records are off
+__global__ void __launch_bounds__(DD_WARPS * 32)
+k_countline_ev(const DDView V, const double* __restrict__ line, int line_per_stream) {
+    DDTlScope tl_(V, 5);
+    const int w = blockIdx.x * DD_WARPS + (threadIdx.x >> 5);
+    if (w >= V.S) return;
+    WarpG g;
+    dd_countline<WarpG, true>(g, V, w, line + (line_per_stream ? (size_t)w * 4 : 0));
+}
+
 // counts [S, C*4] -> out [C*4]; one CTA per output element, tree reduction over streams.
 __global__ void __launch_bounds__(256)
 k_count_reduce(const long long* __restrict__ counts, int S, int n, long long* __restrict__ out,
@@ -363,7 +374,8 @@ static int dd_tick_prepare(const DDView& V, const dd_tracker_config* cfg, int* t
         const void* ks[] = {(const void*)k_prep, (const void*)k_prep_ragged, (const void*)k_gate<true>, (const void*)k_gate<false>,
                             (const void*)k_gallery_stream, (const void*)k_cosine, (const void*)k_match,
                             (const void*)k_match_cta<4>, (const void*)k_match_cta<8>, (const void*)k_apply,
-                            (const void*)k_countline, (const void*)k_count_reduce, (const void*)k_predict};
+                            (const void*)k_countline, (const void*)k_countline_ev, (const void*)k_count_reduce,
+                            (const void*)k_predict};
         for (const void* k : ks)
             if (cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, mx) != cudaSuccess) return DD_ERR_CUDA;
         carve_set = true;
@@ -481,7 +493,13 @@ static int dd_tick_tail(void* state, const dd_tracker_config* cfg, const double*
     DDView V;
     int rc = dd_make_view(state, cfg, &V);
     if (rc != DD_OK) return rc;
-    dd_launch(k_countline, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
+    if (V.ev) {
+        // a new crossing list (a memset node in a captured tick)
+        if (cudaMemsetAsync(V.ev, 0, sizeof(int), st) != cudaSuccess) return DD_ERR_CUDA;
+        dd_launch(k_countline_ev, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
+    } else {
+        dd_launch(k_countline, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
+    }
     DD_CHECK_LAUNCH();
     if (reduce) {
         dd_launch(k_count_reduce, V.C * 4, 256, 0, st, (const long long*)V.counts, V.S, V.C * 4, (long long*)nullptr,

@@ -1048,7 +1048,51 @@ DD_HD int dd_get_label(const DDView& V, size_t slot) {
     return b1;
 }
 
-template <class G>
+// One live track's count-line step (deepdish.py:1046-1112): path point, crossing test, counters.  Returns the counter
+// column its crossing incremented (0 pos, 1 neg; int as well) with its label in *label, or -1.
+DD_HD int dd_countline_track(const DDView& V, size_t slot, double p1x, double p1y, double q1x, double q1y,
+                             long long* cnt, int* label) {
+    if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) return -1;
+    int col = -1;
+    const double* m = V.mean + slot * 8;
+    // Track.to_tlbr (track.py:84-111) and the bottom-centre point (deepdish.py:1060-1063)
+    const double w = dd_mul(m[2], m[3]), h = m[3];
+    const double x = dd_sub(m[0], dd_div(w, 2.0)), y = dd_sub(m[1], dd_div(h, 2.0));
+    const double x2 = dd_add(x, w), y2 = dd_add(y, h);
+    const double bx = dd_div(dd_add(x, x2), 2.0), by = y2;
+    const int n = V.path_n[slot];
+    if (n >= 1) {
+        const double lx = V.path_last[slot * 2], ly = V.path_last[slot * 2 + 1];
+        // p2 = latest, q2 = previous (deepdish.py:1073-1075)
+        const double cp = dd_cross2(dd_sub(q1x, p1x), dd_sub(q1y, p1y), dd_sub(lx, bx), dd_sub(ly, by));
+        if (dd_segments_intersect(p1x, p1y, q1x, q1y, bx, by, lx, ly)) {
+            const int l = dd_get_label(V, slot);
+            if (l >= 0) {
+                col = cp >= 0.0 ? 0 : 1;
+                dd_atomic_add_ll(cnt + l * 4 + col, 1);
+                dd_atomic_add_ll(cnt + l * 4 + 2, 1);
+                *label = l;
+            }
+        }
+        // any_intersection walks the path forwards: segment (previous, latest)
+        if (dd_segments_intersect(p1x, p1y, q1x, q1y, lx, ly, bx, by)) V.path_crossed[slot] = 1;
+    }
+    V.path_last[slot * 2] = bx;
+    V.path_last[slot * 2 + 1] = by;
+    V.path_n[slot] = n + 1;
+    return col;
+}
+
+DD_HD void dd_put_event(const DDView& V, int pos, int s, int track_id, int label, int col) {
+    if (pos >= V.ev_cap) return;                     // overflow: counted in header[0], not written
+    int* r = V.ev + 4 + (size_t)pos * 4;
+    r[0] = s; r[1] = track_id; r[2] = label; r[3] = col;
+}
+
+// EV (config.event_cap > 0, V.ev set): the same counter increments, and one crossing record per increment (layout
+// `events`).  The track loop then runs in warp-uniform rounds: each round's crossings are compacted in order and take
+// their positions with one atomicAdd on header[0], so a stream's records keep the order of tracker.tracks.
+template <class G, bool EV = false>
 DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) {
     const size_t sT = (size_t)s * V.T;
     const double p1x = line[0], p1y = line[1], q1x = line[2], q1y = line[3];
@@ -1058,39 +1102,37 @@ DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) 
     // present tick deleted is not counted a second time
     if (!present) return;
     // deleted tracks (deepdish.py:1041-1044): only the LAST one's result survives the overwrite
+    int del_label = -1, del_id = 0;
     if (g.lane == 0 && ndel > 0) {
         const size_t slot = sT + V.deleted[sT + ndel - 1];
         if (V.path_n[slot] > 1 && V.path_crossed[slot]) {
             const int l = dd_get_label(V, slot);
             if (l >= 0) dd_atomic_add_ll(cnt + l * 4 + 3, 1);
+            if (EV) { del_label = l; del_id = V.track_id[slot]; }
         }
     }
-    for (int t = g.lane; t < nT; t += G::NL) {
-        const size_t slot = sT + V.order[sT + t];
-        if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) continue;
-        const double* m = V.mean + slot * 8;
-        // Track.to_tlbr (track.py:84-111) and the bottom-centre point (deepdish.py:1060-1063)
-        const double w = dd_mul(m[2], m[3]), h = m[3];
-        const double x = dd_sub(m[0], dd_div(w, 2.0)), y = dd_sub(m[1], dd_div(h, 2.0));
-        const double x2 = dd_add(x, w), y2 = dd_add(y, h);
-        const double bx = dd_div(dd_add(x, x2), 2.0), by = y2;
-        const int n = V.path_n[slot];
-        if (n >= 1) {
-            const double lx = V.path_last[slot * 2], ly = V.path_last[slot * 2 + 1];
-            // p2 = latest, q2 = previous (deepdish.py:1073-1075)
-            const double cp = dd_cross2(dd_sub(q1x, p1x), dd_sub(q1y, p1y), dd_sub(lx, bx), dd_sub(ly, by));
-            if (dd_segments_intersect(p1x, p1y, q1x, q1y, bx, by, lx, ly)) {
-                const int l = dd_get_label(V, slot);
-                if (l >= 0) {
-                    dd_atomic_add_ll(cnt + l * 4 + (cp >= 0.0 ? 0 : 1), 1);
-                    dd_atomic_add_ll(cnt + l * 4 + 2, 1);
-                }
-            }
-            // any_intersection walks the path forwards: segment (previous, latest)
-            if (dd_segments_intersect(p1x, p1y, q1x, q1y, lx, ly, bx, by)) V.path_crossed[slot] = 1;
+    if constexpr (!EV) {
+        for (int t = g.lane; t < nT; t += G::NL) {
+            int l;
+            dd_countline_track(V, sT + V.order[sT + t], p1x, p1y, q1x, q1y, cnt, &l);
         }
-        V.path_last[slot * 2] = bx;
-        V.path_last[slot * 2 + 1] = by;
-        V.path_n[slot] = n + 1;
+    } else {
+        for (int t0 = 0; t0 < nT; t0 += G::NL) {
+            const int t = t0 + g.lane;
+            int l = -1, col = -1;
+            size_t slot = 0;
+            if (t < nT) {
+                slot = sT + V.order[sT + t];
+                col = dd_countline_track(V, slot, p1x, p1y, q1x, q1y, cnt, &l);
+            }
+            int total = 0;
+            const int rank = g.scan_excl(col >= 0, total);
+            if (total == 0) continue;
+            int base = 0;
+            if (g.lane == 0) base = dd_atomic_add_i(V.ev, total);
+            base = g.imax(g.lane == 0 ? base : 0);        // lane 0's reservation to every lane (base >= 0)
+            if (col >= 0) dd_put_event(V, base + rank, s, V.track_id[slot], l, col);
+        }
+        if (g.lane == 0 && del_label >= 0) dd_put_event(V, dd_atomic_add_i(V.ev, 1), s, del_id, del_label, 3);
     }
 }

@@ -71,6 +71,8 @@ struct DDView {
     char* segf[DD_MAX_SEGS];         // f32 pages of each pool segment
     char* segh[DD_MAX_SEGS];         // half pages
     int label_rank[DD_MAX_LABELS];
+    int* ev;                         // crossing records: i32 header[4] + [ev_cap][4] (layout `events`), NULL unless
+    int ev_cap;                      // config.event_cap > 0
 };
 
 // ---- gallery pages ----------------------------------------------------------------------------------
@@ -123,6 +125,7 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     if (c->max_tracks > 1024 || c->max_dets > 1024) return DD_ERR_INVALID;
     /* the matching kernel keeps time_since_update in 16-bit shared-memory arrays */
     if (c->max_age < 0 || c->max_age > 32766 || c->n_init < 1) return DD_ERR_INVALID;
+    if (c->event_cap < 0) return DD_ERR_INVALID;
     if (c->seg_pages <= 0 || (c->seg_pages & (c->seg_pages - 1)) != 0) return DD_ERR_INVALID;
     if (c->n_segs < 1 || c->n_segs > DD_MAX_SEGS || c->page_cap < 0) return DD_ERR_INVALID;
     const uint64_t S = c->n_streams, T = c->max_tracks, D = c->max_dets, PT = dd_page_cap(c),
@@ -168,6 +171,7 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     DD_PUT(tick_args, 256);
     DD_PUT(timeline, 8 * 64 * 8 * 2);
     DD_PUT(tick_present, 4 * S);
+    DD_PUT(events, c->event_cap > 0 ? 16 * (1 + (uint64_t)c->event_cap) : 0);     // 0 bytes when off: total_bytes unchanged
 #undef DD_PUT
     L->total_bytes = off;
     return DD_OK;
@@ -211,6 +215,8 @@ static inline int dd_make_view(void* blob, const dd_tracker_config* c, DDView* v
     v->det_feath = (unsigned short*)(b + L.det_feath);
     v->targs = (const DDTickArgs*)(b + L.tick_args);
     v->tl = c->timeline ? (unsigned long long*)(b + L.timeline) : nullptr;
+    v->ev = c->event_cap > 0 ? (int*)(b + L.events) : nullptr;
+    v->ev_cap = c->event_cap;
     v->work = (int*)(b + L.work); v->work_ctl = (int*)(b + L.work_ctl); v->work_rec = (int*)(b + L.work_rec);
     for (int i = 0; i < DD_MAX_SEGS; ++i) {
         const bool on = i < c->n_segs;

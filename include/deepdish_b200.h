@@ -92,7 +92,8 @@ typedef struct dd_tracker_config {
     int32_t gallery_waves;      /* impl 0: 0 = one persistent CTA per SM holding all the triples (default); W > 0 = one
                                    triple per CTA, SMs x triples x W CTAs that each stream a bounded share of the work
                                    list and exit (measured equal on C3, kept as an A/B knob)                         */
-    int32_t reserved0;
+    int32_t event_cap;          /* crossing records kept per tick (count-line events, `events` below); 0 = off: no
+                                   `events` section and the count-line step exactly as without it; < 0 is invalid */
     int32_t timeline;           /* != 0: every tick kernel stamps its first CTA's start and its last CTA's end
                                    (%globaltimer, ns) into the blob's `timeline` words (benchmarks/timeline.py)    */
     uint64_t pool_f32[DD_MAX_SEGS]; /* device pointers, seg_pages x DD_PAGE_F32_BYTES each, 16-byte aligned */
@@ -161,6 +162,16 @@ typedef struct dd_tracker_layout {
                                                   initialises starts to ~0 and ends to 0                         */
     uint64_t tick_present;  /* i32 [S]            1: the stream had a frame in the last tick (written by every tick's
                                                   detection prep; the per-call update marks every stream present)  */
+    uint64_t events;        /* i32 [4 + 4 event_cap] crossing records of the last count-line step, 0 bytes when event_cap = 0
+                                                  (then events == total_bytes).  header[0] = records the step produced (may
+                                                  exceed event_cap: the list overflowed, records past event_cap are counted
+                                                  but not written), header[1..3] unused; then event_cap records
+                                                  {stream (index within this blob), track_id, label, column}, one per counter
+                                                  increment of the step: column 0 / 1 = a live track crossed the line and
+                                                  added 1 to pos / neg and to int of `label` (the label get_label gave the
+                                                  counter), column 3 = the del increment of the last deleted track.  A
+                                                  stream's records keep the order of tracker.tracks, its deletion record
+                                                  last; streams interleave.  Reset at the start of every count-line step */
 } dd_tracker_layout;
 
 /* Host-only arithmetic: fills `host_out`.  No CUDA call. */
@@ -217,7 +228,8 @@ int dd_event_elapsed_ms(void* start, void* end, float* host_ms);   /* both event
 int dd_event_record(void* ev, void* stream);
 
 /* Count-line step (deepdish.py:1035-1114 counting part, :1303-1312; tools/intersection.py:4-30).  Skips a stream
- * that had no frame in the last tick (tick_present; only dd_engine_step_present / _host_present leave one).
+ * that had no frame in the last tick (tick_present; only dd_engine_step_present / _host_present leave one).  With
+ * event_cap > 0 it also lists its crossing records (layout `events`), as every tick's count-line step does.
  *   line f64 [S,4] (x1,y1,x2,y2 per stream) or, with line_per_stream = 0, one f64[4] for all streams. */
 int dd_tracker_countline(void* state, const dd_tracker_config* host_cfg, const double* line,
                          int line_per_stream, void* stream);
@@ -309,6 +321,15 @@ int dd_engine_step_host(void* engine, const void* const* host_blobs, const uint6
  * its blob, which must lie within host_blob_bytes[i].  An absent stream owns no entries of the blob. */
 int dd_engine_step_host_present(void* engine, const void* const* host_blobs, const uint64_t* host_blob_bytes,
                                 const int64_t* host_offsets5, int32_t* host_out_ids, void* caller_stream);
+/* Crossing records of every chunk's latest tick -> host_out (pinned i32): chunk i's block, the 4 + 4 event_cap words of
+ * its `events` section (header, then the records), starts after the blocks of chunks 0 .. i - 1.  Enqueued behind the
+ * chunk's latest tick on a read-back stream of its own, like the det -> track ids of dd_engine_step_host (everything on
+ * caller_stream when n_chunks == 1); the chunk's next tick waits for the copy before its count-line step rewrites the
+ * list, dd_engine_join makes caller_stream wait for it.  Call it right after an engine step (dd_engine_step*): it is
+ * ordered behind the engine's ticks only, so after the per-call path (dd_tracker_countline on a stream of the caller's)
+ * read the `events` section on that stream instead.  DD_ERR_INVALID for a NULL host_out or when a chunk has
+ * event_cap == 0. */
+int dd_engine_copy_events(void* engine, int32_t* host_out, void* caller_stream);
 /* caller_stream waits for every chunk and for the latest count summation (no host synchronisation). */
 int dd_engine_join(void* engine, void* caller_stream);
 /* caller_stream waits for the latest count summation only (total_counts of the last reduced tick). */
