@@ -11,6 +11,7 @@ LIB_PATH = os.path.join(HERE, "libdeepdish_b200.so")
 
 DD_OK, DD_ERR_INVALID, DD_ERR_CUDA, DD_ERR_CAPACITY = 0, -1, -2, -3
 DD_MAX_LABELS = 128
+DD_MAX_LINES = 32
 DD_MAX_SEGS = 16
 PAGE_ROWS, PAGE_F32_BYTES, PAGE_F16_BYTES = 16, 8192, 4096
 FLAG_TRACK_OVERFLOW, FLAG_DET_OVERFLOW, FLAG_LSAP_INFEASIBLE = 1, 2, 4
@@ -29,7 +30,7 @@ class TrackerConfig(ctypes.Structure):
                 ("page_cap", _i32), ("seg_pages", _i32), ("n_segs", _i32),
                 ("gallery_impl", _i32), ("cosine_ctas_per_sm", _i32), ("match_warps", _i32),
                 ("gallery_stages", _i32), ("gallery_waves", _i32), ("event_cap", _i32), ("timeline", _i32),
-                ("pool_f32", _u64 * DD_MAX_SEGS), ("pool_f16", _u64 * DD_MAX_SEGS)]
+                ("n_lines", _i32), ("pool_f32", _u64 * DD_MAX_SEGS), ("pool_f16", _u64 * DD_MAX_SEGS)]
 
 
 LAYOUT_FIELDS = ["n_tracks", "next_id", "n_deleted", "err", "order", "deleted", "counts", "mean", "cov",
@@ -45,6 +46,17 @@ class TrackerLayout(ctypes.Structure):
     _fields_ = [("total_bytes", _u64)] + [(n, _u64) for n in LAYOUT_FIELDS + [EVENTS_FIELD]]
 
 
+def n_lines(cfg):
+    """Count lines per stream (config.n_lines, 0 read as 1)."""
+    return cfg.n_lines or 1
+
+
+def counts_shape(cfg):
+    """Shape of one stream's counters: [C,4] with one count line, [L,C,4] with L > 1."""
+    L = n_lines(cfg)
+    return (cfg.n_labels, 4) if L == 1 else (L, cfg.n_labels, 4)
+
+
 def field_specs(cfg):
     """name -> (dtype string, shape) of every array in the state blob."""
     S, T, D, C = cfg.n_streams, cfg.max_tracks, cfg.max_dets, cfg.n_labels
@@ -53,7 +65,7 @@ def field_specs(cfg):
     i, f, d = "int32", "float32", "float64"
     return {
         "n_tracks": (i, (S,)), "next_id": (i, (S,)), "n_deleted": (i, (S,)), "err": (i, (S,)),
-        "order": (i, (S, T)), "deleted": (i, (S, T)), "counts": ("int64", (S, C, 4)),
+        "order": (i, (S, T)), "deleted": (i, (S, T)), "counts": ("int64", (S,) + counts_shape(cfg)),
         "mean": (d, (S, T, 8)), "cov": (d, (S, T, 8, 8)), "track_id": (i, (S, T)),
         "hits": (i, (S, T)), "age": (i, (S, T)), "tsu": (i, (S, T)), "state": (i, (S, T)),
         "gal_len": (i, (S, T)), "gal_pos": (i, (S, T)), "gal_np": (i, (S, T)), "ptab": (i, (S, T, PT)),
@@ -65,7 +77,7 @@ def field_specs(cfg):
         "work": (i, (S * T,)), "work_ctl": (i, (64,)), "work_rec": (i, (S * T, 16)),
         "det_feath": ("float16", (S, D, 128)), "tick_args": (i, (64,)), "timeline": ("int64", (64, 8, 2)),
         "tick_present": (i, (S,)),
-        # row 0 = header (records this count-line step produced), rows 1.. = {stream, track_id, label, column}
+        # row 0 = header (records this count-line step produced), rows 1.. = {stream, track_id, label, column + 4 line}
         "events": (i, (cfg.event_cap + 1 if cfg.event_cap > 0 else 0, 4)),
     }
 
@@ -79,7 +91,7 @@ def page_cap(cfg):
 def make_config(n_streams, max_tracks, max_dets, budget, labels, max_age=30, n_init=3,
                 max_cosine_distance=0.2, max_iou_distance=0.7, page_cap=0, seg_pages=1024,
                 gallery_impl=0, cosine_ctas_per_sm=0, match_warps=0, gallery_stages=0, gallery_waves=0,
-                timeline=0, event_cap=0):
+                timeline=0, event_cap=0, n_lines=1):
     """Fill a dd_tracker_config from Python values; ``labels`` is the ordered list of label names.
     ``budget=None`` is the reference's nn_budget=None (deepdish.py:515): unbounded galleries (budget 0 in the C
     struct).  The pool segment pointers are filled in by the caller that allocates them."""
@@ -95,7 +107,7 @@ def make_config(n_streams, max_tracks, max_dets, budget, labels, max_age=30, n_i
     cfg.page_cap, cfg.seg_pages, cfg.n_segs = page_cap, seg_pages, 1
     cfg.gallery_impl = GALLERY_IMPLS[gallery_impl] if isinstance(gallery_impl, str) else int(gallery_impl)
     cfg.cosine_ctas_per_sm, cfg.match_warps, cfg.gallery_stages = cosine_ctas_per_sm, match_warps, gallery_stages
-    cfg.gallery_waves, cfg.timeline, cfg.event_cap = gallery_waves, timeline, event_cap
+    cfg.gallery_waves, cfg.timeline, cfg.event_cap, cfg.n_lines = gallery_waves, timeline, event_cap, n_lines
     cfg.feat_dim, cfg.n_labels, cfg.max_age, cfg.n_init = 128, len(labels), max_age, n_init
     cfg.max_cosine_distance, cfg.max_iou_distance = max_cosine_distance, max_iou_distance
     cfg.label_motorbike = labels.index("motorbike") if "motorbike" in labels else -1

@@ -31,6 +31,11 @@ Crossings.__doc__ = """Count-line crossings of one tick, numpy int32 arrays sort
 in the order the reference's ``process_results`` counts them (``tracker.tracks``, then the deleted track): column 0 /
 1 = a live track crossed the line (pos / neg, and int, of ``label``), 3 = the del count of the last deleted track."""
 
+LineCrossings = collections.namedtuple("LineCrossings", "stream track_id label column line")
+LineCrossings.__doc__ = """Crossings of a tracker with several count lines per stream: as ``Crossings``, plus the line each record
+counts on.  Within a stream: ``tracker.tracks`` order, each track's lines ascending, then the deletion records, lines
+ascending."""
+
 
 def _pow2_at_least(n):
     p = 1
@@ -62,7 +67,7 @@ class _Chunk:
                                     gallery_impl=o.gallery_impl, cosine_ctas_per_sm=o.cosine_ctas_per_sm,
                                     match_warps=o.match_warps, gallery_stages=o.gallery_stages,
                                     gallery_waves=o.gallery_waves,
-                                    timeline=o.timeline, event_cap=o.crossing_capacity)
+                                    timeline=o.timeline, event_cap=o.crossing_capacity, n_lines=o.n_lines)
         self.cfgp = ctypes.byref(self.cfg)
         self.segs = []
         for _ in range(n_segs):
@@ -146,7 +151,7 @@ class BatchedTracker:
                  line=None, frame_size=(640, 480), device="cuda", n_chunks=1,
                  pool_pages=None, pool_fraction=0.5, seg_pages=None, page_cap=0,
                  gallery_impl="default", cosine_ctas_per_sm=0, match_warps=0, gallery_stages=0, gallery_waves=0,
-                 timeline=0, gallery_turns=True, engine_graphs=True, crossing_capacity=0):
+                 timeline=0, gallery_turns=True, engine_graphs=True, crossing_capacity=0, lines=None):
         """budget=None is the reference's nn_budget=None (deepdish.py:515-516): galleries grow without bound; the
         page pool and the per-slot page tables are grown between ticks (``maintain``).
 
@@ -155,9 +160,28 @@ class BatchedTracker:
         fewer than 1/8 of the pages are free.  A pool that still runs dry raises in ``check()``.
 
         crossing_capacity > 0: every count-line step also lists its crossings (``crossings()``), up to that many
-        records per chunk and tick; 0 (the default) leaves the count-line step exactly as without it."""
+        records per chunk and tick; 0 (the default) leaves the count-line step exactly as without it.
+
+        Count lines: ``line`` is one segment (x1, y1, x2, y2) for all streams or one per stream ([S,4]); default the
+        reference's vertical mid-line of ``frame_size``.  ``lines`` (instead of ``line``) gives several lines per
+        stream: [L,4] shared by all streams or [S,L,4] per stream, 1 <= L <= 32.  Each line is counted as the reference
+        counts its one line; with L > 1 the counters gain a line axis (``total_counts`` [L,C,4], ``v["counts"]``
+        [S,L,C,4]) and ``crossings()`` returns ``LineCrossings``.  ``lines`` with one line is the tracker ``line=``
+        with that line builds."""
         if int(crossing_capacity) < 0:
             raise ValueError("crossing_capacity must be >= 0")
+        if lines is not None:
+            if line is not None:
+                raise ValueError("give line or lines, not both")
+            lt = torch.as_tensor(lines, dtype=torch.float64)
+            if lt.dim() not in (2, 3) or lt.shape[-1] != 4 or (lt.dim() == 3 and lt.shape[0] != n_streams):
+                raise ValueError("lines: expected [L,4] or [%d,L,4], got %s" % (n_streams, tuple(lt.shape)))
+            if not 1 <= lt.shape[-2] <= _lib.DD_MAX_LINES:
+                raise ValueError("lines: need 1..%d lines per stream, got %d" % (_lib.DD_MAX_LINES, lt.shape[-2]))
+            self.n_lines = int(lt.shape[-2])
+            line = lt[..., 0, :] if self.n_lines == 1 else lt
+        else:
+            self.n_lines = 1
         self.crossing_capacity = int(crossing_capacity)
         self.lib = _lib.lib()
         self.pool_pages, self.pool_fraction, self.seg_pages, self.page_cap = pool_pages, pool_fraction, seg_pages, page_cap
@@ -187,12 +211,13 @@ class BatchedTracker:
             w, h = frame_size
             line = (float(int(w / 2)), 0.0, float(int(w / 2)), float(int(h)))
         lt = torch.as_tensor(line, dtype=torch.float64)
-        self.line_per_stream = 1 if lt.dim() == 2 else 0
+        self.line_per_stream = 1 if lt.dim() == (2 if self.n_lines == 1 else 3) else 0
         self.line = lt.to(self.device).contiguous()
-        S, D, C = n_streams, max_dets, len(self.labels)
+        S, D = n_streams, max_dets
+        cs = _lib.counts_shape(self.cfg)
         self.det_track_id = torch.full((S, D), -1, dtype=torch.int32, device=self.device)
-        self.partial_counts = torch.zeros((2, n_chunks, C, 4), dtype=torch.int64, device=self.device)
-        self.total_counts = torch.zeros((C, 4), dtype=torch.int64, device=self.device)
+        self.partial_counts = torch.zeros((2, n_chunks) + cs, dtype=torch.int64, device=self.device)
+        self.total_counts = torch.zeros(cs, dtype=torch.int64, device=self.device)
         self._tick = 0
         self._aux = torch.cuda.Stream(device=self.device) if n_chunks > 1 else None
         self._poll_pool = any(len(c.segs) * c.cfg.seg_pages < self._worst_pages(c) for c in self.chunks) or budget is None
@@ -355,7 +380,7 @@ class BatchedTracker:
             _lib.check(self.lib.dd_engine_join(self._engine, ctypes.c_void_p(cur.cuda_stream)), "dd_engine_join")
 
     def _line_ptr(self, c):
-        return self.line.data_ptr() + (c.lo * 32 if self.line_per_stream else 0)
+        return self.line.data_ptr() + (c.lo * 32 * self.n_lines if self.line_per_stream else 0)
 
     def _check_batch(self, tlwh, conf, label, feat, count):
         S, D = self.n_streams, self.max_dets
@@ -595,7 +620,8 @@ class BatchedTracker:
                    "dd_engine_copy_events")
 
     def crossings(self, host_buffer=None):
-        """The count-line crossings of the last tick (or per-call ``countline()``) as ``Crossings`` arrays.
+        """The count-line crossings of the last tick (or per-call ``countline()``) as ``Crossings`` arrays
+        (``LineCrossings`` with several lines per stream).
         host_buffer: a buffer a step copied them into (valid once that copy has completed: after join() and a
         synchronisation of the caller's stream); None: read from the device, which joins and synchronises.
         Raises RuntimeError naming the chunk whose list overflowed crossing_capacity (records are never dropped
@@ -620,11 +646,13 @@ class BatchedTracker:
             rec = rec[np.argsort(rec[:, 0], kind="stable")]          # by stream; positions keep the order within one
             parts.append(rec + np.array([c.lo, 0, 0, 0], dtype=np.int32))
         r = np.concatenate(parts).astype(np.int32, copy=False)
+        if self.n_lines > 1:          # column word = column + 4 line
+            return LineCrossings(r[:, 0].copy(), r[:, 1].copy(), r[:, 2].copy(), r[:, 3] & 3, r[:, 3] >> 2)
         return Crossings(r[:, 0].copy(), r[:, 1].copy(), r[:, 2].copy(), r[:, 3].copy())
 
     def reduce_counts(self):
-        """Sum the per-stream counters -> i64 [C,4] (pos, neg, int, del per label), this GPU only.  Runs on the caller's
-        stream, behind every chunk."""
+        """Sum the per-stream counters -> i64 [C,4] (pos, neg, int, del per label; [L,C,4] with L > 1 lines), this GPU
+        only.  Runs on the caller's stream, behind every chunk."""
         self._enter("py")
         self.join()
         sp = ctypes.c_void_p(self._cur().cuda_stream)
@@ -635,7 +663,7 @@ class BatchedTracker:
         return self.total_counts
 
     def all_reduce_counts(self, reduced=False, async_op=False):
-        """[C,4] counters summed over streams and, over NCCL, ranks (the path's only collective).
+        """[C,4] ([L,C,4]) counters summed over streams and, over NCCL, ranks (the path's only collective).
         reduced=True: total_counts already holds this tick's local sum (step(reduce=True) / step_host_packed).
         async_op=True: the all-reduce runs on NCCL's own stream on a copy of the counters (two alternating buffers)
         and the caller's stream is not made to wait, so ranks do not rendezvous every tick; the returned tensor is
@@ -722,9 +750,13 @@ class BatchedTracker:
                 "pools": [[(a.cpu(), b.cpu()) for a, b in c.segs] for c in self.chunks],
                 "page_caps": [_lib.page_cap(c.cfg) for c in self.chunks],
                 "shape": (self.n_streams, self.max_tracks, self.max_dets, self.budget, len(self.labels),
-                          len(self.chunks), self.chunks[0].cfg.seg_pages), "total_counts": self.total_counts.cpu()}
+                          len(self.chunks), self.chunks[0].cfg.seg_pages), "total_counts": self.total_counts.cpu(),
+                "n_lines": self.n_lines}
 
     def load_state_dict(self, sd):
+        if int(sd.get("n_lines", 1)) != self.n_lines:       # checkpoints from before count lines had one line
+            raise ValueError("checkpoint has %d count lines per stream, this tracker %d"
+                             % (int(sd.get("n_lines", 1)), self.n_lines))
         shape = (self.n_streams, self.max_tracks, self.max_dets, self.budget, len(self.labels), len(self.chunks),
                  self.chunks[0].cfg.seg_pages)
         if tuple(sd["shape"]) != shape:

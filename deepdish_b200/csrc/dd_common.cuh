@@ -111,6 +111,17 @@ struct WarpG {
         total = __popc(m);
         return __popc(m & ((1u << lane) - 1u));
     }
+    // exclusive prefix sum of a per-lane count + total (ordered compaction of several items per lane)
+    __device__ int scan_excl_sum(int v, int& total) const {
+        int x = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        total = __shfl_sync(0xffffffffu, x, 31);
+        return x - v;
+    }
     // Warp-wide best key in 3 REDUX ops: min over an order-preserving 64-bit image of the double
     // (hi word, then lo word among the hi-minimal lanes), then max pref among the value-minimal lanes.
     // -0.0 is folded into +0.0 first so that bit equality == IEEE equality (NaN sorts above +inf).
@@ -252,5 +263,6 @@ struct HostG {
     bool any(bool p) const { return p; }
     bool all(bool p) const { return p; }
     int scan_excl(bool p, int& total) const { total = p ? 1 : 0; return 0; }
+    int scan_excl_sum(int v, int& total) const { total = v; return 0; }
     DDKey best(DDKey k) const { return k; }
 };

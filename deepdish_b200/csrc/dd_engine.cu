@@ -67,6 +67,7 @@ struct Chunk {
 
 struct Engine {
     int P = 0, D = 0, C4 = 0, line_per_stream = 0, poll_every = 0;
+    int n_lines = 1;                 // count lines per stream: line is [L,4] or [S,L,4], C4 = L * C * 4
     bool turns = false;              // chunks take turns on the gallery stream (see dd_engine_create)
     bool graphs = true;              // replay captured graphs (dd_engine_set_graphs(0): launch the tick's kernels plainly)
     cudaEvent_t last_gal = nullptr;  // end of the most recently enqueued gallery stream
@@ -101,7 +102,7 @@ void drop_graphs(Chunk& c) {
 }
 
 int capture_piece(Engine& E, Chunk& c, int ragged, int reduce, int parts, cudaGraphExec_t* out) {
-    const double* line = E.line + (E.line_per_stream ? (size_t)c.lo * 4 : 0);
+    const double* line = E.line + (E.line_per_stream ? (size_t)c.lo * E.n_lines * 4 : 0);
     DD_CU(cudaStreamBeginCapture(E.cap, cudaStreamCaptureModeRelaxed));
     const int rc = dd_capture_tick(c.state, &c.cfg, ragged, reduce, parts, line, E.line_per_stream, E.cap);
     cudaGraph_t g = nullptr;
@@ -147,7 +148,7 @@ int launch_tick(Engine& E, Chunk& c, const DDTickArgs& A, int ragged, int reduce
     int rc = E.graphs ? ensure_graphs(E, c, ragged, reduce) : dd_tick_prepare_host(c.state, &c.cfg);
     if (rc != DD_OK) return rc;
     cudaGraphExec_t* g = c.graph[ragged][reduce];
-    const double* line = E.line + (E.line_per_stream ? (size_t)c.lo * 4 : 0);
+    const double* line = E.line + (E.line_per_stream ? (size_t)c.lo * E.n_lines * 4 : 0);
     // one piece of the tick behind the prep kernel: its captured graph, or the same kernels launched plainly (they read
     // the tick's inputs through tick_args either way)
     auto piece = [&](int k, int parts) -> int {
@@ -251,8 +252,8 @@ int dd_engine_create(int32_t n_chunks, void* const* host_states, const dd_tracke
         c.n = c.cfg.n_streams;
         c.events_off = L.events;
         c.st = n_chunks > 1 ? (cudaStream_t)host_streams[i] : nullptr;
-        if (i == 0) { E->D = c.cfg.max_dets; E->C4 = c.cfg.n_labels * 4; }
-        ok = c.cfg.max_dets == E->D && c.cfg.n_labels * 4 == E->C4 &&
+        if (i == 0) { E->D = c.cfg.max_dets; E->n_lines = dd_n_lines(&c.cfg); E->C4 = E->n_lines * c.cfg.n_labels * 4; }
+        ok = c.cfg.max_dets == E->D && dd_n_lines(&c.cfg) == E->n_lines && E->n_lines * c.cfg.n_labels * 4 == E->C4 &&
              cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&c.copied, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&c.copied2, cudaEventDisableTiming) == cudaSuccess &&

@@ -6,7 +6,8 @@
 //   gallery kernel persistent grid over the work list     <- the HBM-bound kernel (dd_gallery.cuh)
 //   k_match        stream -> 1 warp (4 / 8 for crowds)    cascade + IoU stage + lifecycle, dynamic shared memory
 //   k_apply        (stream, detection) -> 8 lanes         Kalman update / initiate + gallery append + label vote
-//   k_countline    stream -> 1 warp                       (k_countline_ev: + the crossing records)
+//   k_countline    stream -> 1 warp                       (k_countline_ev: + the crossing records; k_countline_lines:
+//                                                         several count lines per stream)
 //   k_count_reduce one CTA per counter
 #include <cuda_runtime.h>
 #include "dd_gallery.cuh"
@@ -234,7 +235,26 @@ k_countline_ev(const DDView V, const double* __restrict__ line, int line_per_str
     dd_countline<WarpG, true>(g, V, w, line + (line_per_stream ? (size_t)w * 4 : 0));
 }
 
-// counts [S, C*4] -> out [C*4]; one CTA per output element, tree reduction over streams.
+// Several count lines per stream (config.n_lines > 1; EV: + the crossing records): separate kernels, so that k_countline
+// and k_countline_ev stay exactly what they are with one line.  Each warp stages its stream's L lines in shared memory
+// (DD_WARPS x L x 4 doubles) once, instead of re-reading them for every track.
+template <bool EV>
+__global__ void __launch_bounds__(DD_WARPS * 32)
+k_countline_lines(const DDView V, const double* __restrict__ line, int line_per_stream) {
+    DDTlScope tl_(V, 5);
+    extern __shared__ __align__(16) char smem_lines[];
+    const int w = blockIdx.x * DD_WARPS + (threadIdx.x >> 5);
+    if (w >= V.S) return;
+    WarpG g;
+    const int n = V.n_lines * 4;
+    double* mine = (double*)smem_lines + (threadIdx.x >> 5) * n;
+    const double* src = line + (line_per_stream ? (size_t)w * n : 0);
+    for (int i = g.lane; i < n; i += 32) mine[i] = src[i];
+    __syncwarp();
+    dd_countline_lines<WarpG, EV>(g, V, w, mine);
+}
+
+// counts [S, L*C*4] -> out [L*C*4]; one CTA per output element, tree reduction over streams.
 __global__ void __launch_bounds__(256)
 k_count_reduce(const long long* __restrict__ counts, int S, int n, long long* __restrict__ out,
                const DDTickArgs* __restrict__ ind) {
@@ -374,8 +394,8 @@ static int dd_tick_prepare(const DDView& V, const dd_tracker_config* cfg, int* t
         const void* ks[] = {(const void*)k_prep, (const void*)k_prep_ragged, (const void*)k_gate<true>, (const void*)k_gate<false>,
                             (const void*)k_gallery_stream, (const void*)k_cosine, (const void*)k_match,
                             (const void*)k_match_cta<4>, (const void*)k_match_cta<8>, (const void*)k_apply,
-                            (const void*)k_countline, (const void*)k_countline_ev, (const void*)k_count_reduce,
-                            (const void*)k_predict};
+                            (const void*)k_countline, (const void*)k_countline_ev, (const void*)k_countline_lines<false>,
+                            (const void*)k_countline_lines<true>, (const void*)k_count_reduce, (const void*)k_predict};
         for (const void* k : ks)
             if (cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, mx) != cudaSuccess) return DD_ERR_CUDA;
         carve_set = true;
@@ -493,16 +513,23 @@ static int dd_tick_tail(void* state, const dd_tracker_config* cfg, const double*
     DDView V;
     int rc = dd_make_view(state, cfg, &V);
     if (rc != DD_OK) return rc;
-    if (V.ev) {
-        // a new crossing list (a memset node in a captured tick)
-        if (cudaMemsetAsync(V.ev, 0, sizeof(int), st) != cudaSuccess) return DD_ERR_CUDA;
+    // a new crossing list (a memset node in a captured tick)
+    if (V.ev && cudaMemsetAsync(V.ev, 0, sizeof(int), st) != cudaSuccess) return DD_ERR_CUDA;
+    if (V.n_lines > 1) {
+        const size_t sm = (size_t)DD_WARPS * V.n_lines * 4 * sizeof(double);
+        if (V.ev)
+            dd_launch(k_countline_lines<true>, warps_to_blocks(V.S), DD_WARPS * 32, sm, st, V, line, line_per_stream);
+        else
+            dd_launch(k_countline_lines<false>, warps_to_blocks(V.S), DD_WARPS * 32, sm, st, V, line, line_per_stream);
+    } else if (V.ev) {
         dd_launch(k_countline_ev, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
     } else {
         dd_launch(k_countline, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
     }
     DD_CHECK_LAUNCH();
     if (reduce) {
-        dd_launch(k_count_reduce, V.C * 4, 256, 0, st, (const long long*)V.counts, V.S, V.C * 4, (long long*)nullptr,
+        const int n = V.n_lines * V.C * 4;
+        dd_launch(k_count_reduce, n, 256, 0, st, (const long long*)V.counts, V.S, n, (long long*)nullptr,
                   (const DDTickArgs*)V.targs);
         DD_CHECK_LAUNCH();
     }
@@ -724,7 +751,8 @@ int dd_tracker_count_reduce(void* state, const dd_tracker_config* cfg, int64_t* 
     int rc = dd_make_view(state, cfg, &V);
     if (rc != DD_OK) return rc;
     if (!out_counts) return DD_ERR_INVALID;
-    k_count_reduce<<<V.C * 4, 256, 0, (cudaStream_t)stream>>>(V.counts, V.S, V.C * 4, (long long*)out_counts, nullptr);
+    const int n = V.n_lines * V.C * 4;
+    k_count_reduce<<<n, 256, 0, (cudaStream_t)stream>>>(V.counts, V.S, n, (long long*)out_counts, nullptr);
     DD_CHECK_LAUNCH();
     return DD_OK;
 }

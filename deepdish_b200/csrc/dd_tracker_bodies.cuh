@@ -7,6 +7,7 @@
 //   dd_match_stream    (stream)         matching cascade + IoU stage + track lifecycle
 //   dd_apply_det       (stream, det)    Kalman update / initiate + gallery append + label vote
 //   dd_countline       (stream)         count-line crossing + per-label counters
+//   dd_countline_lines (stream)         the same for several count lines per stream (config.n_lines > 1)
 #pragma once
 #include "dd_view.h"
 #include "dd_kalman.cuh"
@@ -1134,5 +1135,120 @@ DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) 
             if (col >= 0) dd_put_event(V, base + rank, s, V.track_id[slot], l, col);
         }
         if (g.lane == 0 && del_label >= 0) dd_put_event(V, dd_atomic_add_i(V.ev, 1), s, del_id, del_label, 3);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Several count lines per stream (config.n_lines = L > 1).  Line l is counted into counts[s][l] exactly as the
+// reference's process_results counts its one line; dd_countline above stays the one-line step.
+// ------------------------------------------------------------------------------------------------
+// One live track's step against the stream's L lines (lines[4 l ..] = x1, y1, x2, y2): the bottom-centre point once,
+// each line's crossing and direction test against the previous point, get_label once if some line was crossed, the
+// path_crossed bits and the path point once.  Returns the mask of the lines whose counters it incremented (bit l), with
+// the neg direction of each in *neg (bit l set: column 1, else 0) and its label in *label.
+DD_HD unsigned dd_countline_track_lines(const DDView& V, size_t slot, const double* lines, long long* cnt,
+                                        unsigned* neg, int* label) {
+    if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) return 0u;
+    unsigned hit = 0u;
+    const double* m = V.mean + slot * 8;
+    const double w = dd_mul(m[2], m[3]), h = m[3];
+    const double x = dd_sub(m[0], dd_div(w, 2.0)), y = dd_sub(m[1], dd_div(h, 2.0));
+    const double x2 = dd_add(x, w), y2 = dd_add(y, h);
+    const double bx = dd_div(dd_add(x, x2), 2.0), by = y2;
+    const int n = V.path_n[slot];
+    if (n >= 1) {
+        const double lx = V.path_last[slot * 2], ly = V.path_last[slot * 2 + 1];
+        unsigned ng = 0u, crossed = 0u;
+        for (int l = 0; l < V.n_lines; ++l) {
+            const double p1x = lines[l * 4], p1y = lines[l * 4 + 1], q1x = lines[l * 4 + 2], q1y = lines[l * 4 + 3];
+            if (dd_segments_intersect(p1x, p1y, q1x, q1y, bx, by, lx, ly)) {
+                const double cp = dd_cross2(dd_sub(q1x, p1x), dd_sub(q1y, p1y), dd_sub(lx, bx), dd_sub(ly, by));
+                hit |= 1u << l;
+                if (!(cp >= 0.0)) ng |= 1u << l;
+            }
+            if (dd_segments_intersect(p1x, p1y, q1x, q1y, lx, ly, bx, by)) crossed |= 1u << l;
+        }
+        if (hit) {
+            const int lab = dd_get_label(V, slot);
+            if (lab >= 0) {
+                for (int l = 0; l < V.n_lines; ++l) {
+                    if (!((hit >> l) & 1u)) continue;
+                    long long* c = cnt + ((size_t)l * V.C + lab) * 4;
+                    dd_atomic_add_ll(c + ((ng >> l) & 1u), 1);
+                    dd_atomic_add_ll(c + 2, 1);
+                }
+                *neg = ng;
+                *label = lab;
+            } else {
+                hit = 0u;
+            }
+        }
+        if (crossed) V.path_crossed[slot] |= (int)crossed;
+    }
+    V.path_last[slot * 2] = bx;
+    V.path_last[slot * 2 + 1] = by;
+    V.path_n[slot] = n + 1;
+    return hit;
+}
+
+// dd_countline for L lines; `lines` = the stream's [L,4] segments (the kernel stages them in shared memory).  EV: one
+// record per counter increment, column word = column + 4 line.  A lane writes up to L records in a round, so the
+// round's records are placed with a warp prefix sum of the per-lane counts: a stream's records follow tracker.tracks,
+// each track's lines ascending, then the deletion records, lines ascending.
+template <class G, bool EV = false>
+DD_HD void dd_countline_lines(const G& g, const DDView& V, int s, const double* lines) {
+    const size_t sT = (size_t)s * V.T;
+    long long* cnt = V.counts + (size_t)s * V.n_lines * V.C * 4;
+    const int present = V.tick_present[s], ndel = V.n_deleted[s], nT = V.n_tracks[s];
+    if (!present) return;
+    // deleted tracks (deepdish.py:1041-1044): only the LAST one's result survives the overwrite, on every line whose
+    // bit its path set
+    int del_label = -1, del_id = 0;
+    unsigned del_lines = 0u;
+    if (g.lane == 0 && ndel > 0) {
+        const size_t slot = sT + V.deleted[sT + ndel - 1];
+        const unsigned crossed = (unsigned)V.path_crossed[slot];
+        if (V.path_n[slot] > 1 && crossed) {
+            const int l = dd_get_label(V, slot);
+            if (l >= 0)
+                for (int k = 0; k < V.n_lines; ++k)
+                    if ((crossed >> k) & 1u) dd_atomic_add_ll(cnt + ((size_t)k * V.C + l) * 4 + 3, 1);
+            if (EV) { del_label = l; del_id = V.track_id[slot]; del_lines = crossed; }
+        }
+    }
+    if constexpr (!EV) {
+        for (int t = g.lane; t < nT; t += G::NL) {
+            unsigned ng;
+            int l;
+            dd_countline_track_lines(V, sT + V.order[sT + t], lines, cnt, &ng, &l);
+        }
+    } else {
+        for (int t0 = 0; t0 < nT; t0 += G::NL) {
+            const int t = t0 + g.lane;
+            unsigned hit = 0u, ng = 0u;
+            int l = -1;
+            size_t slot = 0;
+            if (t < nT) {
+                slot = sT + V.order[sT + t];
+                hit = dd_countline_track_lines(V, slot, lines, cnt, &ng, &l);
+            }
+            int total = 0;
+            const int rank = g.scan_excl_sum(dd_popc(hit), total);
+            if (total == 0) continue;
+            int base = 0;
+            if (g.lane == 0) base = dd_atomic_add_i(V.ev, total);
+            base = g.imax(g.lane == 0 ? base : 0);        // lane 0's reservation to every lane (base >= 0)
+            if (hit) {
+                int pos = base + rank;
+                const int tid = V.track_id[slot];
+                for (int k = 0; k < V.n_lines; ++k)
+                    if ((hit >> k) & 1u) dd_put_event(V, pos++, s, tid, l, (int)((ng >> k) & 1u) + 4 * k);
+            }
+        }
+        if (g.lane == 0 && del_label >= 0) {
+            int pos = dd_atomic_add_i(V.ev, dd_popc(del_lines));
+            for (int k = 0; k < V.n_lines; ++k)
+                if ((del_lines >> k) & 1u) dd_put_event(V, pos++, s, del_id, del_label, 3 + 4 * k);
+        }
     }
 }

@@ -73,6 +73,7 @@ struct DDView {
     int label_rank[DD_MAX_LABELS];
     int* ev;                         // crossing records: i32 header[4] + [ev_cap][4] (layout `events`), NULL unless
     int ev_cap;                      // config.event_cap > 0
+    int n_lines;                     // count lines per stream (counts [S,n_lines,C,4])
 };
 
 // ---- gallery pages ----------------------------------------------------------------------------------
@@ -117,6 +118,9 @@ static inline int dd_page_cap(const dd_tracker_config* c) {
     return c->page_cap > need ? c->page_cap : need;
 }
 
+// config.n_lines, 0 read as 1 (zero-initialised configs)
+static inline int dd_n_lines(const dd_tracker_config* c) { return c->n_lines == 0 ? 1 : c->n_lines; }
+
 static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layout* L) {
     if (!c || !L) return DD_ERR_INVALID;
     if (c->n_streams <= 0 || c->max_tracks <= 0 || c->max_dets <= 0 || c->budget < 0) return DD_ERR_INVALID;
@@ -126,10 +130,11 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     /* the matching kernel keeps time_since_update in 16-bit shared-memory arrays */
     if (c->max_age < 0 || c->max_age > 32766 || c->n_init < 1) return DD_ERR_INVALID;
     if (c->event_cap < 0) return DD_ERR_INVALID;
+    if (dd_n_lines(c) < 1 || dd_n_lines(c) > DD_MAX_LINES) return DD_ERR_INVALID;
     if (c->seg_pages <= 0 || (c->seg_pages & (c->seg_pages - 1)) != 0) return DD_ERR_INVALID;
     if (c->n_segs < 1 || c->n_segs > DD_MAX_SEGS || c->page_cap < 0) return DD_ERR_INVALID;
     const uint64_t S = c->n_streams, T = c->max_tracks, D = c->max_dets, PT = dd_page_cap(c),
-                   C = c->n_labels, F = DD_FEAT_DIM, DW = (D + 31) / 32;
+                   C = c->n_labels, F = DD_FEAT_DIM, DW = (D + 31) / 32, NLN = dd_n_lines(c);
     uint64_t off = 0;
 #define DD_PUT(name, bytes) do { L->name = off; off = dd_align256(off + (uint64_t)(bytes)); } while (0)
     DD_PUT(n_tracks, 4 * S);
@@ -138,7 +143,7 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     DD_PUT(err, 4 * S);
     DD_PUT(order, 4 * S * T);
     DD_PUT(deleted, 4 * S * T);
-    DD_PUT(counts, 8 * S * C * 4);
+    DD_PUT(counts, 8 * S * NLN * C * 4);
     DD_PUT(mean, 8 * S * T * 8);
     DD_PUT(cov, 8 * S * T * 64);
     DD_PUT(track_id, 4 * S * T);
@@ -217,6 +222,7 @@ static inline int dd_make_view(void* blob, const dd_tracker_config* c, DDView* v
     v->tl = c->timeline ? (unsigned long long*)(b + L.timeline) : nullptr;
     v->ev = c->event_cap > 0 ? (int*)(b + L.events) : nullptr;
     v->ev_cap = c->event_cap;
+    v->n_lines = dd_n_lines(c);
     v->work = (int*)(b + L.work); v->work_ctl = (int*)(b + L.work_ctl); v->work_rec = (int*)(b + L.work_rec);
     for (int i = 0; i < DD_MAX_SEGS; ++i) {
         const bool on = i < c->n_segs;

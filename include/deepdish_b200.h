@@ -30,6 +30,7 @@ extern "C" {
 #define DD_ERR_CAPACITY  (-3)   /* T > max_tracks or D > max_dets: never silently truncated          */
 
 #define DD_MAX_LABELS   128
+#define DD_MAX_LINES    32      /* count lines per stream (dd_tracker_config.n_lines)                */
 #define DD_FEAT_DIM     128     /* MARS re-ID feature width (tools/generate_detections.py:137-140)   */
 
 /* track states, deep_sort/track.py:15-17 (0 = slot unused) */
@@ -96,6 +97,8 @@ typedef struct dd_tracker_config {
                                    `events` section and the count-line step exactly as without it; < 0 is invalid */
     int32_t timeline;           /* != 0: every tick kernel stamps its first CTA's start and its last CTA's end
                                    (%globaltimer, ns) into the blob's `timeline` words (benchmarks/timeline.py)    */
+    int32_t n_lines;            /* L: count lines per stream, 1..DD_MAX_LINES (0 = 1).  Each line is counted as the
+                                   reference's process_results counts its one line; `counts` holds L counter sets  */
     uint64_t pool_f32[DD_MAX_SEGS]; /* device pointers, seg_pages x DD_PAGE_F32_BYTES each, 16-byte aligned */
     uint64_t pool_f16[DD_MAX_SEGS]; /* device pointers, seg_pages x DD_PAGE_F16_BYTES each, 16-byte aligned */
 } dd_tracker_config;
@@ -115,7 +118,7 @@ typedef struct dd_tracker_layout {
     uint64_t err;           /* i32 [S]            DD_FLAG_* bits                                    */
     uint64_t order;         /* i32 [S,Tmax]       slot of the k-th live track (creation order)      */
     uint64_t deleted;       /* i32 [S,Tmax]       slots deleted by the last update (creation order) */
-    uint64_t counts;        /* i64 [S,C,4]        pos, neg, int, del per label                      */
+    uint64_t counts;        /* i64 [S,L,C,4]      pos, neg, int, del per line and label (L = n_lines) */
     /* per slot */
     uint64_t mean;          /* f64 [S,Tmax,8]                                                       */
     uint64_t cov;           /* f64 [S,Tmax,8,8]                                                     */
@@ -138,7 +141,7 @@ typedef struct dd_tracker_layout {
     uint64_t lab_sum;       /* f64 [S,Tmax,C]     sum of confidences per label                      */
     uint64_t path_n;        /* i32 [S,Tmax]       points in the count-line path db                  */
     uint64_t path_last;     /* f64 [S,Tmax,2]     last bottom-centre point                          */
-    uint64_t path_crossed;  /* i32 [S,Tmax]       any path segment crossed the line                 */
+    uint64_t path_crossed;  /* i32 [S,Tmax]       bit l: a path segment crossed line l (0 / 1 when L = 1) */
     /* per-tick scratch / outputs */
     uint64_t gate;          /* u32 [S,Tmax,ceil(Dmax/32)]  bit d set: d^2 <= chi2inv95[4]           */
     uint64_t cost;          /* f32 [S,Tmax,Dmax]  min cosine distance (valid where gate bit set)    */
@@ -166,12 +169,14 @@ typedef struct dd_tracker_layout {
                                                   (then events == total_bytes).  header[0] = records the step produced (may
                                                   exceed event_cap: the list overflowed, records past event_cap are counted
                                                   but not written), header[1..3] unused; then event_cap records
-                                                  {stream (index within this blob), track_id, label, column}, one per counter
-                                                  increment of the step: column 0 / 1 = a live track crossed the line and
-                                                  added 1 to pos / neg and to int of `label` (the label get_label gave the
-                                                  counter), column 3 = the del increment of the last deleted track.  A
-                                                  stream's records keep the order of tracker.tracks, its deletion record
-                                                  last; streams interleave.  Reset at the start of every count-line step */
+                                                  {stream (index within this blob), track_id, label, column + 4 line}, one
+                                                  per counter increment of the step: column 0 / 1 = a live track crossed
+                                                  line `line` and added 1 to pos / neg and to int of `label` (the label
+                                                  get_label gave the counter), column 3 = the del increment of the last
+                                                  deleted track (line is 0 when L = 1).  A stream's records keep the order
+                                                  of tracker.tracks, each track's lines ascending, then its deletion
+                                                  records, lines ascending; streams interleave.  Reset at the start of
+                                                  every count-line step */
 } dd_tracker_layout;
 
 /* Host-only arithmetic: fills `host_out`.  No CUDA call. */
@@ -230,7 +235,8 @@ int dd_event_record(void* ev, void* stream);
 /* Count-line step (deepdish.py:1035-1114 counting part, :1303-1312; tools/intersection.py:4-30).  Skips a stream
  * that had no frame in the last tick (tick_present; only dd_engine_step_present / _host_present leave one).  With
  * event_cap > 0 it also lists its crossing records (layout `events`), as every tick's count-line step does.
- *   line f64 [S,4] (x1,y1,x2,y2 per stream) or, with line_per_stream = 0, one f64[4] for all streams. */
+ *   line f64 [S,L,4] (x1,y1,x2,y2 per stream and line, L = n_lines) or, with line_per_stream = 0, one f64 [L,4] for
+ *   all streams.  Each line l is counted into counts[s][l] exactly as the reference counts its one line. */
 int dd_tracker_countline(void* state, const dd_tracker_config* host_cfg, const double* line,
                          int line_per_stream, void* stream);
 
@@ -245,7 +251,7 @@ int dd_unpack_detections(const void* blob, int32_t n_streams, int32_t max_dets, 
                          int64_t off_label, int64_t off_feat, double* det_tlwh, float* det_conf,
                          int32_t* det_label, float* det_feat, int32_t* det_count, void* stream);
 
-/* Sum the per-stream counters into out_counts i64 [C,4] (the tensor handed to the NCCL all-reduce). */
+/* Sum the per-stream counters into out_counts i64 [L,C,4] (the tensor handed to the NCCL all-reduce). */
 int dd_tracker_count_reduce(void* state, const dd_tracker_config* host_cfg, int64_t* out_counts,
                             void* stream);
 
@@ -266,7 +272,8 @@ int dd_tracker_status(void* state, const dd_tracker_config* host_cfg, int32_t* h
 /*   host_states[i], host_cfgs[i]  blob and config of chunk i (configs are copied), host_first_stream[i] its first stream;
  *   host_streams[i]               the chunk's CUDA stream, aux_stream the summation stream (both ignored -- everything runs
  *                                 on the caller's stream -- when n_chunks == 1);
- *   line f64 [4] or [S,4]; partial_counts i64 [2,n_chunks,C,4]; total_counts i64 [C,4]; det_track_id i32 [S,Dmax];
+ *   line f64 [L,4] or [S,L,4] (as dd_tracker_countline); partial_counts i64 [2,n_chunks,L,C,4]; total_counts i64 [L,C,4];
+ *   det_track_id i32 [S,Dmax]; every chunk must have the same max_dets, n_labels and n_lines;
  *   poll_every > 0: every that many ticks the chunk's pool counters are copied to pinned memory behind its tick
  *   (dd_engine_pool_latest reads them without synchronising);
  *   gallery_turns != 0 (n_chunks > 1): the chunks take turns on the HBM-bound gallery stream -- each one waits for the
