@@ -111,16 +111,17 @@ struct WarpG {
         total = __popc(m);
         return __popc(m & ((1u << lane) - 1u));
     }
-    // exclusive prefix sum of a per-lane count + total (ordered compaction of several items per lane)
-    __device__ int scan_excl_sum(int v, int& total) const {
-        int x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
+    // exclusive prefix sum of a per-lane count 0 <= v < 2^bits + total (ordered compaction of several items per lane):
+    // one ballot per bit, so counts of 0 / 1 cost what scan_excl costs
+    __device__ int scan_excl_sum(int v, int bits, int& total) const {
+        int rank = 0;
+        total = 0;
+        for (int b = 0; b < bits; ++b) {
+            const unsigned m = __ballot_sync(0xffffffffu, (v >> b) & 1);
+            total += __popc(m) << b;
+            rank += __popc(m & ((1u << lane) - 1u)) << b;
         }
-        total = __shfl_sync(0xffffffffu, x, 31);
-        return x - v;
+        return rank;
     }
     // Warp-wide best key in 3 REDUX ops: min over an order-preserving 64-bit image of the double
     // (hi word, then lo word among the hi-minimal lanes), then max pref among the value-minimal lanes.
@@ -263,6 +264,6 @@ struct HostG {
     bool any(bool p) const { return p; }
     bool all(bool p) const { return p; }
     int scan_excl(bool p, int& total) const { total = p ? 1 : 0; return 0; }
-    int scan_excl_sum(int v, int& total) const { total = v; return 0; }
+    int scan_excl_sum(int v, int, int& total) const { total = v; return 0; }
     DDKey best(DDKey k) const { return k; }
 };

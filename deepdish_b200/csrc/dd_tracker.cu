@@ -6,8 +6,7 @@
 //   gallery kernel persistent grid over the work list     <- the HBM-bound kernel (dd_gallery.cuh)
 //   k_match        stream -> 1 warp (4 / 8 for crowds)    cascade + IoU stage + lifecycle, dynamic shared memory
 //   k_apply        (stream, detection) -> 8 lanes         Kalman update / initiate + gallery append + label vote
-//   k_countline    stream -> 1 warp                       (k_countline_ev: + the crossing records; k_countline_lines:
-//                                                         several count lines per stream)
+//   k_countline    stream -> 1 warp                       config.n_lines lines (EV: + the crossing records)
 //   k_count_reduce one CTA per counter
 #include <cuda_runtime.h>
 #include "dd_gallery.cuh"
@@ -215,43 +214,15 @@ k_apply(const DDView V, const DDTickArgs A) {
     dd_apply_det(g, V, w / V.D, w % V.D, det_conf, det_label, scratch[threadIdx.x / DD_SUB]);
 }
 
+// Count-line step, one warp per stream (EV: + the crossing records, config.event_cap > 0).
+template <bool EV>
 __global__ void __launch_bounds__(DD_WARPS * 32)
 k_countline(const DDView V, const double* __restrict__ line, int line_per_stream) {
     DDTlScope tl_(V, 5);
     const int w = blockIdx.x * DD_WARPS + (threadIdx.x >> 5);
     if (w >= V.S) return;
     WarpG g;
-    dd_countline(g, V, w, line + (line_per_stream ? (size_t)w * 4 : 0));
-}
-
-// k_countline that also writes the crossing records (config.event_cap > 0); a kernel of its own so that k_countline
-// stays exactly what it is when the records are off
-__global__ void __launch_bounds__(DD_WARPS * 32)
-k_countline_ev(const DDView V, const double* __restrict__ line, int line_per_stream) {
-    DDTlScope tl_(V, 5);
-    const int w = blockIdx.x * DD_WARPS + (threadIdx.x >> 5);
-    if (w >= V.S) return;
-    WarpG g;
-    dd_countline<WarpG, true>(g, V, w, line + (line_per_stream ? (size_t)w * 4 : 0));
-}
-
-// Several count lines per stream (config.n_lines > 1; EV: + the crossing records): separate kernels, so that k_countline
-// and k_countline_ev stay exactly what they are with one line.  Each warp stages its stream's L lines in shared memory
-// (DD_WARPS x L x 4 doubles) once, instead of re-reading them for every track.
-template <bool EV>
-__global__ void __launch_bounds__(DD_WARPS * 32)
-k_countline_lines(const DDView V, const double* __restrict__ line, int line_per_stream) {
-    DDTlScope tl_(V, 5);
-    extern __shared__ __align__(16) char smem_lines[];
-    const int w = blockIdx.x * DD_WARPS + (threadIdx.x >> 5);
-    if (w >= V.S) return;
-    WarpG g;
-    const int n = V.n_lines * 4;
-    double* mine = (double*)smem_lines + (threadIdx.x >> 5) * n;
-    const double* src = line + (line_per_stream ? (size_t)w * n : 0);
-    for (int i = g.lane; i < n; i += 32) mine[i] = src[i];
-    __syncwarp();
-    dd_countline_lines<WarpG, EV>(g, V, w, mine);
+    dd_countline<WarpG, EV>(g, V, w, line + (line_per_stream ? (size_t)w * V.n_lines * 4 : 0));
 }
 
 // counts [S, L*C*4] -> out [L*C*4]; one CTA per output element, tree reduction over streams.
@@ -394,8 +365,8 @@ static int dd_tick_prepare(const DDView& V, const dd_tracker_config* cfg, int* t
         const void* ks[] = {(const void*)k_prep, (const void*)k_prep_ragged, (const void*)k_gate<true>, (const void*)k_gate<false>,
                             (const void*)k_gallery_stream, (const void*)k_cosine, (const void*)k_match,
                             (const void*)k_match_cta<4>, (const void*)k_match_cta<8>, (const void*)k_apply,
-                            (const void*)k_countline, (const void*)k_countline_ev, (const void*)k_countline_lines<false>,
-                            (const void*)k_countline_lines<true>, (const void*)k_count_reduce, (const void*)k_predict};
+                            (const void*)k_countline<false>, (const void*)k_countline<true>, (const void*)k_count_reduce,
+                            (const void*)k_predict};
         for (const void* k : ks)
             if (cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, mx) != cudaSuccess) return DD_ERR_CUDA;
         carve_set = true;
@@ -515,17 +486,10 @@ static int dd_tick_tail(void* state, const dd_tracker_config* cfg, const double*
     if (rc != DD_OK) return rc;
     // a new crossing list (a memset node in a captured tick)
     if (V.ev && cudaMemsetAsync(V.ev, 0, sizeof(int), st) != cudaSuccess) return DD_ERR_CUDA;
-    if (V.n_lines > 1) {
-        const size_t sm = (size_t)DD_WARPS * V.n_lines * 4 * sizeof(double);
-        if (V.ev)
-            dd_launch(k_countline_lines<true>, warps_to_blocks(V.S), DD_WARPS * 32, sm, st, V, line, line_per_stream);
-        else
-            dd_launch(k_countline_lines<false>, warps_to_blocks(V.S), DD_WARPS * 32, sm, st, V, line, line_per_stream);
-    } else if (V.ev) {
-        dd_launch(k_countline_ev, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
-    } else {
-        dd_launch(k_countline, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
-    }
+    if (V.ev)
+        dd_launch(k_countline<true>, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
+    else
+        dd_launch(k_countline<false>, warps_to_blocks(V.S), DD_WARPS * 32, 0, st, V, line, line_per_stream);
     DD_CHECK_LAUNCH();
     if (reduce) {
         const int n = V.n_lines * V.C * 4;

@@ -6,8 +6,7 @@
 //   dd_cosine_track    (stream, track)  gallery min cosine distance for the gate-passing pairs
 //   dd_match_stream    (stream)         matching cascade + IoU stage + track lifecycle
 //   dd_apply_det       (stream, det)    Kalman update / initiate + gallery append + label vote
-//   dd_countline       (stream)         count-line crossing + per-label counters
-//   dd_countline_lines (stream)         the same for several count lines per stream (config.n_lines > 1)
+//   dd_countline       (stream)         count-line crossings (config.n_lines lines) + per-line, per-label counters
 #pragma once
 #include "dd_view.h"
 #include "dd_kalman.cuh"
@@ -1049,12 +1048,19 @@ DD_HD int dd_get_label(const DDView& V, size_t slot) {
     return b1;
 }
 
-// One live track's count-line step (deepdish.py:1046-1112): path point, crossing test, counters.  Returns the counter
-// column its crossing incremented (0 pos, 1 neg; int as well) with its label in *label, or -1.
-DD_HD int dd_countline_track(const DDView& V, size_t slot, double p1x, double p1y, double q1x, double q1y,
-                             long long* cnt, int* label) {
-    if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) return -1;
-    int col = -1;
+// ------------------------------------------------------------------------------------------------
+// Count-line step (deepdish.py:1035-1114) against the stream's L = config.n_lines >= 1 lines: line l is counted into
+// counts[s][l] exactly as the reference's process_results counts its one line.
+// ------------------------------------------------------------------------------------------------
+// One live track's step (deepdish.py:1046-1112) against the L lines (lines[4 l ..] = x1, y1, x2, y2): the
+// bottom-centre point once, each line's crossing and direction test against the previous point, get_label once if
+// some line was crossed, the path_crossed bits and the path point once.  Returns the mask of the lines whose counters
+// it incremented (bit l), with the neg direction of each in *neg (bit l set: column 1, else column 0) and its label in
+// *label.
+DD_HD unsigned dd_countline_track(const DDView& V, size_t slot, const double* lines, long long* cnt, unsigned* neg,
+                                  int* label) {
+    if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) return 0u;
+    unsigned hit = 0u;
     const double* m = V.mean + slot * 8;
     // Track.to_tlbr (track.py:84-111) and the bottom-centre point (deepdish.py:1060-1063)
     const double w = dd_mul(m[2], m[3]), h = m[3];
@@ -1064,108 +1070,17 @@ DD_HD int dd_countline_track(const DDView& V, size_t slot, double p1x, double p1
     const int n = V.path_n[slot];
     if (n >= 1) {
         const double lx = V.path_last[slot * 2], ly = V.path_last[slot * 2 + 1];
-        // p2 = latest, q2 = previous (deepdish.py:1073-1075)
-        const double cp = dd_cross2(dd_sub(q1x, p1x), dd_sub(q1y, p1y), dd_sub(lx, bx), dd_sub(ly, by));
-        if (dd_segments_intersect(p1x, p1y, q1x, q1y, bx, by, lx, ly)) {
-            const int l = dd_get_label(V, slot);
-            if (l >= 0) {
-                col = cp >= 0.0 ? 0 : 1;
-                dd_atomic_add_ll(cnt + l * 4 + col, 1);
-                dd_atomic_add_ll(cnt + l * 4 + 2, 1);
-                *label = l;
-            }
-        }
-        // any_intersection walks the path forwards: segment (previous, latest)
-        if (dd_segments_intersect(p1x, p1y, q1x, q1y, lx, ly, bx, by)) V.path_crossed[slot] = 1;
-    }
-    V.path_last[slot * 2] = bx;
-    V.path_last[slot * 2 + 1] = by;
-    V.path_n[slot] = n + 1;
-    return col;
-}
-
-DD_HD void dd_put_event(const DDView& V, int pos, int s, int track_id, int label, int col) {
-    if (pos >= V.ev_cap) return;                     // overflow: counted in header[0], not written
-    int* r = V.ev + 4 + (size_t)pos * 4;
-    r[0] = s; r[1] = track_id; r[2] = label; r[3] = col;
-}
-
-// EV (config.event_cap > 0, V.ev set): the same counter increments, and one crossing record per increment (layout
-// `events`).  The track loop then runs in warp-uniform rounds: each round's crossings are compacted in order and take
-// their positions with one atomicAdd on header[0], so a stream's records keep the order of tracker.tracks.
-template <class G, bool EV = false>
-DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* line) {
-    const size_t sT = (size_t)s * V.T;
-    const double p1x = line[0], p1y = line[1], q1x = line[2], q1y = line[3];
-    long long* cnt = V.counts + (size_t)s * V.C * 4;
-    const int present = V.tick_present[s], ndel = V.n_deleted[s], nT = V.n_tracks[s];
-    // a stream without a frame in the last tick takes no count-line step: in particular the last track its previous
-    // present tick deleted is not counted a second time
-    if (!present) return;
-    // deleted tracks (deepdish.py:1041-1044): only the LAST one's result survives the overwrite
-    int del_label = -1, del_id = 0;
-    if (g.lane == 0 && ndel > 0) {
-        const size_t slot = sT + V.deleted[sT + ndel - 1];
-        if (V.path_n[slot] > 1 && V.path_crossed[slot]) {
-            const int l = dd_get_label(V, slot);
-            if (l >= 0) dd_atomic_add_ll(cnt + l * 4 + 3, 1);
-            if (EV) { del_label = l; del_id = V.track_id[slot]; }
-        }
-    }
-    if constexpr (!EV) {
-        for (int t = g.lane; t < nT; t += G::NL) {
-            int l;
-            dd_countline_track(V, sT + V.order[sT + t], p1x, p1y, q1x, q1y, cnt, &l);
-        }
-    } else {
-        for (int t0 = 0; t0 < nT; t0 += G::NL) {
-            const int t = t0 + g.lane;
-            int l = -1, col = -1;
-            size_t slot = 0;
-            if (t < nT) {
-                slot = sT + V.order[sT + t];
-                col = dd_countline_track(V, slot, p1x, p1y, q1x, q1y, cnt, &l);
-            }
-            int total = 0;
-            const int rank = g.scan_excl(col >= 0, total);
-            if (total == 0) continue;
-            int base = 0;
-            if (g.lane == 0) base = dd_atomic_add_i(V.ev, total);
-            base = g.imax(g.lane == 0 ? base : 0);        // lane 0's reservation to every lane (base >= 0)
-            if (col >= 0) dd_put_event(V, base + rank, s, V.track_id[slot], l, col);
-        }
-        if (g.lane == 0 && del_label >= 0) dd_put_event(V, dd_atomic_add_i(V.ev, 1), s, del_id, del_label, 3);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Several count lines per stream (config.n_lines = L > 1).  Line l is counted into counts[s][l] exactly as the
-// reference's process_results counts its one line; dd_countline above stays the one-line step.
-// ------------------------------------------------------------------------------------------------
-// One live track's step against the stream's L lines (lines[4 l ..] = x1, y1, x2, y2): the bottom-centre point once,
-// each line's crossing and direction test against the previous point, get_label once if some line was crossed, the
-// path_crossed bits and the path point once.  Returns the mask of the lines whose counters it incremented (bit l), with
-// the neg direction of each in *neg (bit l set: column 1, else 0) and its label in *label.
-DD_HD unsigned dd_countline_track_lines(const DDView& V, size_t slot, const double* lines, long long* cnt,
-                                        unsigned* neg, int* label) {
-    if (V.state[slot] != DD_STATE_CONFIRMED || V.tsu[slot] > 1) return 0u;
-    unsigned hit = 0u;
-    const double* m = V.mean + slot * 8;
-    const double w = dd_mul(m[2], m[3]), h = m[3];
-    const double x = dd_sub(m[0], dd_div(w, 2.0)), y = dd_sub(m[1], dd_div(h, 2.0));
-    const double x2 = dd_add(x, w), y2 = dd_add(y, h);
-    const double bx = dd_div(dd_add(x, x2), 2.0), by = y2;
-    const int n = V.path_n[slot];
-    if (n >= 1) {
-        const double lx = V.path_last[slot * 2], ly = V.path_last[slot * 2 + 1];
+        const unsigned was = (unsigned)V.path_crossed[slot];     // read beside the path, off the counters' chain
         unsigned ng = 0u, crossed = 0u;
         for (int l = 0; l < V.n_lines; ++l) {
             const double p1x = lines[l * 4], p1y = lines[l * 4 + 1], q1x = lines[l * 4 + 2], q1y = lines[l * 4 + 3];
+            // p2 = latest, q2 = previous (deepdish.py:1073-1075)
             if (dd_segments_intersect(p1x, p1y, q1x, q1y, bx, by, lx, ly)) {
                 const double cp = dd_cross2(dd_sub(q1x, p1x), dd_sub(q1y, p1y), dd_sub(lx, bx), dd_sub(ly, by));
                 hit |= 1u << l;
                 if (!(cp >= 0.0)) ng |= 1u << l;
             }
+            // any_intersection walks the path forwards: segment (previous, latest)
             if (dd_segments_intersect(p1x, p1y, q1x, q1y, lx, ly, bx, by)) crossed |= 1u << l;
         }
         if (hit) {
@@ -1183,7 +1098,7 @@ DD_HD unsigned dd_countline_track_lines(const DDView& V, size_t slot, const doub
                 hit = 0u;
             }
         }
-        if (crossed) V.path_crossed[slot] |= (int)crossed;
+        if (crossed) V.path_crossed[slot] = (int)(was | crossed);
     }
     V.path_last[slot * 2] = bx;
     V.path_last[slot * 2 + 1] = by;
@@ -1191,15 +1106,25 @@ DD_HD unsigned dd_countline_track_lines(const DDView& V, size_t slot, const doub
     return hit;
 }
 
-// dd_countline for L lines; `lines` = the stream's [L,4] segments (the kernel stages them in shared memory).  EV: one
-// record per counter increment, column word = column + 4 line.  A lane writes up to L records in a round, so the
-// round's records are placed with a warp prefix sum of the per-lane counts: a stream's records follow tracker.tracks,
-// each track's lines ascending, then the deletion records, lines ascending.
+DD_HD void dd_put_event(const DDView& V, int pos, int s, int track_id, int label, int col) {
+    if (pos >= V.ev_cap) return;                     // overflow: counted in header[0], not written
+    int* r = V.ev + 4 + (size_t)pos * 4;
+    r[0] = s; r[1] = track_id; r[2] = label; r[3] = col;
+}
+
+// The stream's step; `lines` = its [L,4] segments.  EV (config.event_cap > 0, V.ev set): the same counter increments,
+// and one crossing record per increment (layout `events`), column word = column + 4 line.  The track loop then runs in
+// warp-uniform rounds; a lane writes up to L records in a round, so the round's records are placed with a warp prefix
+// sum of the per-lane counts (one ballot per bit of L: a single one when L = 1) and take their positions with one
+// atomicAdd on header[0]: a stream's records follow tracker.tracks, each track's lines ascending, then the deletion
+// records (column 3), lines ascending.
 template <class G, bool EV = false>
-DD_HD void dd_countline_lines(const G& g, const DDView& V, int s, const double* lines) {
+DD_HD void dd_countline(const G& g, const DDView& V, int s, const double* lines) {
     const size_t sT = (size_t)s * V.T;
     long long* cnt = V.counts + (size_t)s * V.n_lines * V.C * 4;
     const int present = V.tick_present[s], ndel = V.n_deleted[s], nT = V.n_tracks[s];
+    // a stream without a frame in the last tick takes no count-line step: in particular the last track its previous
+    // present tick deleted is not counted a second time
     if (!present) return;
     // deleted tracks (deepdish.py:1041-1044): only the LAST one's result survives the overwrite, on every line whose
     // bit its path set
@@ -1220,9 +1145,11 @@ DD_HD void dd_countline_lines(const G& g, const DDView& V, int s, const double* 
         for (int t = g.lane; t < nT; t += G::NL) {
             unsigned ng;
             int l;
-            dd_countline_track_lines(V, sT + V.order[sT + t], lines, cnt, &ng, &l);
+            dd_countline_track(V, sT + V.order[sT + t], lines, cnt, &ng, &l);
         }
     } else {
+        int bits = 0;                                     // of the per-lane record count, at most L
+        for (int k = V.n_lines; k; k >>= 1) ++bits;
         for (int t0 = 0; t0 < nT; t0 += G::NL) {
             const int t = t0 + g.lane;
             unsigned hit = 0u, ng = 0u;
@@ -1230,10 +1157,10 @@ DD_HD void dd_countline_lines(const G& g, const DDView& V, int s, const double* 
             size_t slot = 0;
             if (t < nT) {
                 slot = sT + V.order[sT + t];
-                hit = dd_countline_track_lines(V, slot, lines, cnt, &ng, &l);
+                hit = dd_countline_track(V, slot, lines, cnt, &ng, &l);
             }
             int total = 0;
-            const int rank = g.scan_excl_sum(dd_popc(hit), total);
+            const int rank = g.scan_excl_sum(dd_popc(hit), bits, total);
             if (total == 0) continue;
             int base = 0;
             if (g.lane == 0) base = dd_atomic_add_i(V.ev, total);

@@ -79,13 +79,53 @@ int ddh_gallery_read(void* state, const dd_tracker_config* cfg, int s, int slot_
     return n;
 }
 
-int ddh_tracker_countline(void* state, const dd_tracker_config* cfg, const double* line,
-                          int line_per_stream) {
+// The count-line step as dd_tick_tail issues it: a new crossing list when the records are on, then the step of every
+// stream.  lines f64 [S,L,4].
+static void ddh_countline_step(const DDView& V, const double* lines) {
+    HostG g;
+    if (V.ev) V.ev[0] = 0;
+    for (int s = 0; s < V.S; ++s) {
+        const double* l = lines + (size_t)s * V.n_lines * 4;
+        if (V.ev)
+            dd_countline<HostG, true>(g, V, s, l);
+        else
+            dd_countline<HostG, false>(g, V, s, l);
+    }
+}
+
+int ddh_tracker_countline(void* state, const dd_tracker_config* cfg, const double* lines) {
+    DDView V;
+    int rc = dd_make_view(state, cfg, &V);
+    if (rc != DD_OK) return rc;
+    ddh_countline_step(V, lines);
+    return DD_OK;
+}
+
+// One fused tick as the engine runs it (k_prep, k_gate<true>, gallery, k_match, k_apply, k_countline), with frame
+// presence.  present u8 [S] (NULL = every stream present); lines f64 [S,L,4].
+int ddh_tracker_tick(void* state, const dd_tracker_config* cfg, const double* det_tlwh, const float* det_conf,
+                     const int32_t* det_label, const float* det_feat, const int32_t* det_count, const uint8_t* present,
+                     const double* lines, int32_t* out_det_track_id) {
     DDView V;
     int rc = dd_make_view(state, cfg, &V);
     if (rc != DD_OK) return rc;
     HostG g;
-    for (int s = 0; s < V.S; ++s) dd_countline(g, V, s, line + (line_per_stream ? (size_t)s * 4 : 0));
+    for (int s = 0; s < V.S; ++s)
+        for (int d = 0; d < V.D; ++d) dd_prep_det(g, V, s, d, det_tlwh, det_feat, det_count, present);
+    for (int s = 0; s < V.S; ++s)
+        for (int t = 0; t < V.T; ++t) {
+            dd_tick_predict_track(g, V, s, t);
+            dd_gate_track(g, V, s, t, det_count);
+        }
+    for (int s = 0; s < V.S; ++s)
+        for (int t = 0; t < V.T; ++t) { DDDirectPass<HostG> pass; dd_cosine_track(g, V, s, t, det_count, pass); }
+    std::vector<char> smem(dd_match_smem_bytes(V.T, V.D, V.tab_cap) + 16);
+    for (int s = 0; s < V.S; ++s)
+        dd_match_stream(g, V, s, det_tlwh, det_count, out_det_track_id, smem.data());
+    double scratch[64];
+    for (int s = 0; s < V.S; ++s)
+        for (int d = 0; d < V.D; ++d) dd_apply_det(g, V, s, d, det_conf, det_label, scratch);
+    ddh_countline_step(V, lines);
     return DD_OK;
 }
 

@@ -43,7 +43,10 @@ class HostEmuTracker:
             n = int(np.prod(shape)) * np.dtype(dt).itemsize
             self.v[name] = self.blob[off:off + n].view(dt).reshape(shape)
         assert emu().ddh_tracker_init(_p(self.blob), ctypes.byref(cfg)) == 0
-        self.line = np.asarray(line, dtype=np.float64)
+        # the count lines as f64 [S,L,4]: line [4] / [L,4] (every stream) or [S,L,4] (per stream)
+        n = L.n_lines(cfg)
+        self.line = np.ascontiguousarray(np.broadcast_to(np.asarray(line, np.float64).reshape(-1, n, 4),
+                                                         (cfg.n_streams, n, 4)))
         self.det_track_id = np.zeros((cfg.n_streams, cfg.max_dets), dtype=np.int32)
 
     def predict(self):
@@ -66,8 +69,28 @@ class HostEmuTracker:
         assert got == n
         return out[:n]
 
+    def tick(self, tlwh, conf, label, feat, count, present=None):
+        """predict + update + count-line in one tick, as the engine runs it; present: u8-like [S] (None: every
+        stream present)."""
+        self._keep = [np.ascontiguousarray(tlwh, np.float64), np.ascontiguousarray(conf, np.float32),
+                      np.ascontiguousarray(label, np.int32), np.ascontiguousarray(feat, np.float32),
+                      np.ascontiguousarray(count, np.int32)]
+        pr = None if present is None else np.ascontiguousarray(np.asarray(present).astype(np.uint8))
+        a = self._keep
+        rc = emu().ddh_tracker_tick(_p(self.blob), ctypes.byref(self.cfg), _p(a[0]), _p(a[1]), _p(a[2]), _p(a[3]),
+                                    _p(a[4]), _p(pr) if pr is not None else None, _p(self.line),
+                                    _p(self.det_track_id))
+        assert rc == 0
+        return self.det_track_id
+
     def countline(self):
-        assert emu().ddh_tracker_countline(_p(self.blob), ctypes.byref(self.cfg), _p(self.line), 0) == 0
+        assert emu().ddh_tracker_countline(_p(self.blob), ctypes.byref(self.cfg), _p(self.line)) == 0
+
+    def events(self):
+        """(records of the last count-line step, the rows written: int32 [min(n, cap), 4])."""
+        ev = self.v["events"]
+        n = int(ev[0, 0])
+        return n, ev[1:1 + min(n, self.cfg.event_cap)].copy()
 
 
 def lsap(cost):

@@ -1,5 +1,5 @@
-"""Crossing records on the CPU: the count-line body k_countline_ev runs, compiled with a one-lane group, lists one
-record per counter increment -- live crossings in tracker.tracks order, then the deletion record -- exactly as the
+"""Crossing records on the CPU: the count-line body k_countline<true> runs, compiled with a one-lane group, lists
+one record per counter increment -- live crossings in tracker.tracks order, then the deletion record -- exactly as the
 oracle's process_results counts them, tick by tick, across frame-presence drops; an overflowing list counts every
 record and writes the first event_cap."""
 import numpy as np
@@ -8,7 +8,7 @@ import pytest
 from deepdish_b200 import _lib as L
 from tests import crossings as X
 from tests import presence as P
-from tests.hostemu.crossings import HostEmuCrossingsTracker
+from tests.hostemu.driver import HostEmuTracker
 from tests.parity import compare_stream
 
 
@@ -18,8 +18,8 @@ def scene():
 
 
 def _emu(cap):
-    return HostEmuCrossingsTracker(L.make_config(X.S, X.T, X.DMAX, P.BUDGET, X.LABELS, max_age=P.MAX_AGE,
-                                                 event_cap=cap), line=X.LINE)
+    return HostEmuTracker(L.make_config(X.S, X.T, X.DMAX, P.BUDGET, X.LABELS, max_age=P.MAX_AGE, event_cap=cap),
+                          line=X.LINE)
 
 
 def _tick(emu, b, p):

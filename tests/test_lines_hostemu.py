@@ -1,4 +1,4 @@
-"""Several count lines per camera on the CPU: the count-line body k_countline_lines runs, compiled with a one-lane group,
+"""Several count lines per camera on the CPU: the count-line body k_countline runs, compiled with a one-lane group,
 counts every line of every stream exactly as an oracle LineCounter of that line counts it, tick by tick, across
 frame-presence drops; with records on it lists them merged in the device's order (tracker.tracks, each track's lines
 ascending, then the deletion records, lines ascending) and an overflowing list counts every record and writes the first
@@ -11,7 +11,7 @@ from deepdish_b200 import _lib as L
 from tests import crossings as X
 from tests import lines as LN
 from tests import presence as P
-from tests.hostemu.lines import HostEmuLinesTracker
+from tests.hostemu.driver import HostEmuTracker
 from tests.parity import compare_stream
 
 
@@ -22,8 +22,8 @@ def scene():
 
 def _emu(scene, cap):
     n = scene.lines.shape[1]
-    return HostEmuLinesTracker(L.make_config(X.S, X.T, X.DMAX, P.BUDGET, X.LABELS, max_age=P.MAX_AGE, event_cap=cap,
-                                             n_lines=n), scene.lines)
+    return HostEmuTracker(L.make_config(X.S, X.T, X.DMAX, P.BUDGET, X.LABELS, max_age=P.MAX_AGE, event_cap=cap,
+                                        n_lines=n), line=scene.lines)
 
 
 def _tick(emu, b, p):

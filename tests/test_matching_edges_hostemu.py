@@ -6,7 +6,7 @@ import pytest
 
 from deepdish_b200 import _lib as L
 from tests import matching_edges as M
-from tests.hostemu.tick import HostEmuTickTracker
+from tests.hostemu.driver import HostEmuTracker
 from tests.parity import LABELS3
 
 FUZZ_SEEDS = tuple(range(40))
@@ -18,7 +18,7 @@ class _Emu:
     def __init__(self, S, T, D, max_age, cos, iou, per_call=False):
         cfg = L.make_config(S, T, D, M.BUDGET, LABELS3, max_age=max_age, max_cosine_distance=cos,
                             max_iou_distance=iou)
-        self.emu, self.per_call = HostEmuTickTracker(cfg), per_call
+        self.emu, self.per_call = HostEmuTracker(cfg), per_call
 
     def tick(self, b):
         a = (b.tlwh.numpy(), b.conf.numpy(), b.label.numpy(), b.feat.numpy(), b.count.numpy())

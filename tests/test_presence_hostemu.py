@@ -5,7 +5,7 @@ import pytest
 
 from deepdish_b200 import _lib as L
 from tests import presence as P
-from tests.hostemu.tick import HostEmuTickTracker
+from tests.hostemu.driver import HostEmuTracker
 from tests.parity import compare_stream, LABELS3
 
 
@@ -15,7 +15,7 @@ def scene():
 
 
 def _emu():
-    return HostEmuTickTracker(L.make_config(P.S, 48, P.DMAX, P.BUDGET, LABELS3, max_age=P.MAX_AGE))
+    return HostEmuTracker(L.make_config(P.S, 48, P.DMAX, P.BUDGET, LABELS3, max_age=P.MAX_AGE))
 
 
 def _tick(emu, b, present):
