@@ -13,6 +13,7 @@ DD_OK, DD_ERR_INVALID, DD_ERR_CUDA, DD_ERR_CAPACITY = 0, -1, -2, -3
 DD_MAX_LABELS = 128
 DD_MAX_LINES = 32
 DD_MAX_SEGS = 16
+SMEM_OPTIN_BYTES = 227 * 1024     # DD_SMEM_OPTIN_BYTES (csrc/dd_view.h): the matching step's shared memory must fit it
 PAGE_ROWS, PAGE_F32_BYTES, PAGE_F16_BYTES = 16, 8192, 4096
 FLAG_TRACK_OVERFLOW, FLAG_DET_OVERFLOW, FLAG_LSAP_INFEASIBLE = 1, 2, 4
 FLAG_POOL_EXHAUSTED, FLAG_GALLERY_OVERFLOW, FLAG_BAD_LABEL = 8, 16, 32
@@ -116,6 +117,26 @@ def make_config(n_streams, max_tracks, max_dets, budget, labels, max_age=30, n_i
     for k, n in enumerate(labels):
         cfg.label_rank[k] = ranks[n]
     return cfg
+
+
+def check_shape(L, max_tracks, max_dets):
+    """Raise ValueError, before any CUDA work, when the layout query of library L rejects (max_tracks, max_dets): each
+    is at most 1024 and together they must leave the matching step within SMEM_OPTIN_BYTES of shared memory."""
+    def fits(d):
+        cfg = make_config(1, max_tracks, d, None, ["x"])
+        return L.dd_tracker_layout_query(ctypes.byref(cfg), ctypes.byref(TrackerLayout())) == DD_OK
+    if fits(max_dets):
+        return
+    if max_dets < 1 or not fits(1):
+        raise ValueError("max_tracks must be in 1..1024 and max_dets >= 1, got max_tracks=%d, max_dets=%d"
+                         % (max_tracks, max_dets))
+    lo, hi = 1, max_dets               # fits(lo), not fits(hi): the layout only grows with max_dets
+    while hi - lo > 1:
+        mid = (lo + hi) // 2
+        lo, hi = (mid, hi) if fits(mid) else (lo, mid)
+    raise ValueError("max_tracks=%d, max_dets=%d: max_dets is at most 1024, and the matching step's shared memory must "
+                     "fit %d bytes (227 KB) a block; the largest max_dets that fits max_tracks=%d is %d"
+                     % (max_tracks, max_dets, SMEM_OPTIN_BYTES, max_tracks, lo))
 
 
 _lib = None

@@ -153,7 +153,11 @@ class BatchedTracker:
                  gallery_impl="default", cosine_ctas_per_sm=0, match_warps=0, gallery_stages=0, gallery_waves=0,
                  timeline=0, gallery_turns=True, engine_graphs=True, crossing_capacity=0, lines=None):
         """budget=None is the reference's nn_budget=None (deepdish.py:515-516): galleries grow without bound; the
-        page pool and the per-slot page tables are grown between ticks (``maintain``).
+        page pool and the per-slot page tables are grown between ticks (``maintain``).  budget=0 is the same, as
+        nn_budget=0 keeps every sample in the reference (``samples[-0:]``).
+
+        max_tracks and max_dets are each at most 1024, and together they must leave the matching step within 227 KB of
+        shared memory (max_tracks 1024: max_dets <= 992); a shape that does not fit raises ValueError here.
 
         Gallery memory: ``pool_pages`` 16-row pages per chunk (default: ``pool_fraction`` of the worst case
         streams x max_tracks x ceil(budget / 16)), in segments of ``seg_pages``; more segments are attached when
@@ -184,6 +188,9 @@ class BatchedTracker:
             self.n_lines = 1
         self.crossing_capacity = int(crossing_capacity)
         self.lib = _lib.lib()
+        _lib.check_shape(self.lib, max_tracks, max_dets)
+        if budget == 0:
+            budget = None
         self.pool_pages, self.pool_fraction, self.seg_pages, self.page_cap = pool_pages, pool_fraction, seg_pages, page_cap
         self.gallery_impl, self.cosine_ctas_per_sm, self.match_warps = gallery_impl, cosine_ctas_per_sm, match_warps
         self.gallery_stages, self.gallery_waves = gallery_stages, gallery_waves

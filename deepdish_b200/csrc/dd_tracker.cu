@@ -344,10 +344,10 @@ static void dd_launch(void (*kernel)(KArgs...), unsigned grid, unsigned block, s
 // Function attributes (opt-in shared memory) are set here, outside any stream capture.
 static int dd_tick_prepare(const DDView& V, const dd_tracker_config* cfg, int* triples_out, int* stages_out, int* mw_out) {
     const size_t smem = dd_match_smem_bytes(V.T, V.D, V.tab_cap);
-    if (smem > 227 * 1024) return DD_ERR_INVALID;
+    if (smem > DD_SMEM_OPTIN_BYTES) return DD_ERR_INVALID;     // dd_layout_compute rejects such a layout first
     int mw = cfg->match_warps;
     if (mw != 1 && mw != 4 && mw != 8) mw = (V.T > 160 || V.D > 160) ? 4 : 1;
-    if (mw > 1 && smem + 256 > 227 * 1024) mw = 1;
+    if (mw > 1 && smem + 256 > DD_SMEM_OPTIN_BYTES) mw = 1;
     // Function attributes belong to a device: the caches below (what has been opted in so far; the attributes only ever
     // grow) are kept per device, so a process that drives several GPUs sets them on each.
     struct Opted { size_t match = 0, cta = 0, gsm = 0; bool carve = false; };

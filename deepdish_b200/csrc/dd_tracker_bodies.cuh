@@ -409,31 +409,11 @@ struct DDMatchSmem {
 // Three regions are never live at the same time and share one union: the gate words + staged costs (matching cascade
 // only), the three CPython-set tables (set-order step between the cascade and the IoU stage) and tbox (IoU stage
 // only).  The matching warp's shared memory decides how many streams fit on an SM beside another chunk's gallery
-// stream, so every kilobyte here is occupancy.
-#ifndef DD_CVAL
-#define DD_CVAL 4       // gate-passing costs per track kept in shared memory (the rest is read from global)
-#endif
+// stream, so every kilobyte here is occupancy.  The sizes (dd_match_smem_bytes) are in dd_view.h, whose layout check
+// rejects a configuration whose matching step does not fit.
 #ifndef DD_MB
 #define DD_MB 4         // iterations per batch of the matching warp's staging loops (loads first, then stores)
 #endif
-DD_HD size_t dd_match_union_bytes(int T, int D, int tab_cap) {
-    const size_t a = (size_t)T * ((D + 31) / 32) * 4 + (size_t)T * DD_CVAL * 4;
-    const size_t b = (size_t)tab_cap * 2 * 3;
-    const size_t c = (size_t)T * 5 * 8;
-    size_t m = a > b ? a : b;
-    m = m > c ? m : c;
-    return (m + 15) & ~(size_t)15;
-}
-DD_HD size_t dd_match_smem_base_bytes(int T, int D, int tab_cap) {
-    const int n = T > D ? T : D;
-    size_t b = dd_lsap_scratch_bytes(n);
-    b += (size_t)T * 2 * 6 + (size_t)D * 2 * 2 + (size_t)n * 2 * 2;
-    b += (size_t)T * 2;
-    return (b + 15) & ~(size_t)15;
-}
-DD_HD size_t dd_match_smem_bytes(int T, int D, int tab_cap) {
-    return dd_match_smem_base_bytes(T, D, tab_cap) + (size_t)D * 32 + dd_match_union_bytes(T, D, tab_cap) + 16;
-}
 
 DD_HD void dd_match_carve(char* mem, int T, int D, int tab_cap, DDMatchSmem& m) {
     const int n = T > D ? T : D;

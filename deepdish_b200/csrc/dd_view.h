@@ -121,6 +121,32 @@ static inline int dd_page_cap(const dd_tracker_config* c) {
 // config.n_lines, 0 read as 1 (zero-initialised configs)
 static inline int dd_n_lines(const dd_tracker_config* c) { return c->n_lines == 0 ? 1 : c->n_lines; }
 
+// Shared memory of the matching step of one stream (the plan is drawn at DDMatchSmem, dd_tracker_bodies.cuh).  It grows
+// with T and D together, so the layout check below rejects every (max_tracks, max_dets) whose matching step cannot
+// launch, and the tick's own check (dd_tick_prepare) uses the same sizes and limit.
+#define DD_SMEM_OPTIN_BYTES (227 * 1024)   // opt-in dynamic shared memory of one CTA (sm_100)
+#ifndef DD_CVAL
+#define DD_CVAL 4       // gate-passing costs per track kept in shared memory (the rest is read from global)
+#endif
+DD_HD size_t dd_match_union_bytes(int T, int D, int tab_cap) {
+    const size_t a = (size_t)T * ((D + 31) / 32) * 4 + (size_t)T * DD_CVAL * 4;
+    const size_t b = (size_t)tab_cap * 2 * 3;
+    const size_t c = (size_t)T * 5 * 8;
+    size_t m = a > b ? a : b;
+    m = m > c ? m : c;
+    return (m + 15) & ~(size_t)15;
+}
+DD_HD size_t dd_match_smem_base_bytes(int T, int D, int tab_cap) {
+    const int n = T > D ? T : D;
+    size_t b = dd_lsap_scratch_bytes(n);
+    b += (size_t)T * 2 * 6 + (size_t)D * 2 * 2 + (size_t)n * 2 * 2;
+    b += (size_t)T * 2;
+    return (b + 15) & ~(size_t)15;
+}
+DD_HD size_t dd_match_smem_bytes(int T, int D, int tab_cap) {
+    return dd_match_smem_base_bytes(T, D, tab_cap) + (size_t)D * 32 + dd_match_union_bytes(T, D, tab_cap) + 16;
+}
+
 static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layout* L) {
     if (!c || !L) return DD_ERR_INVALID;
     if (c->n_streams <= 0 || c->max_tracks <= 0 || c->max_dets <= 0 || c->budget < 0) return DD_ERR_INVALID;
@@ -133,6 +159,8 @@ static inline int dd_layout_compute(const dd_tracker_config* c, dd_tracker_layou
     if (dd_n_lines(c) < 1 || dd_n_lines(c) > DD_MAX_LINES) return DD_ERR_INVALID;
     if (c->seg_pages <= 0 || (c->seg_pages & (c->seg_pages - 1)) != 0) return DD_ERR_INVALID;
     if (c->n_segs < 1 || c->n_segs > DD_MAX_SEGS || c->page_cap < 0) return DD_ERR_INVALID;
+    if (dd_match_smem_bytes(c->max_tracks, c->max_dets, dd_set_table_slots(c->max_tracks)) > DD_SMEM_OPTIN_BYTES)
+        return DD_ERR_INVALID;
     const uint64_t S = c->n_streams, T = c->max_tracks, D = c->max_dets, PT = dd_page_cap(c),
                    C = c->n_labels, F = DD_FEAT_DIM, DW = (D + 31) / 32, NLN = dd_n_lines(c);
     uint64_t off = 0;

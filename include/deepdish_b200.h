@@ -63,8 +63,11 @@ const char* dd_version(void);
  * ---------------------------------------------------------------------------------------------- */
 typedef struct dd_tracker_config {
     int32_t n_streams;          /* S                                                                */
-    int32_t max_tracks;         /* Tmax: slots per stream (live + deleted-this-tick + new)          */
-    int32_t max_dets;           /* Dmax: detections per stream per tick                             */
+    int32_t max_tracks;         /* Tmax: slots per stream (live + deleted-this-tick + new), <= 1024 */
+    int32_t max_dets;           /* Dmax: detections per stream per tick, <= 1024.  The limit is joint:
+                                   the matching step's shared memory grows with Tmax and Dmax together
+                                   and must fit 227 KB (Tmax 1024: Dmax <= 992; Tmax <= 991: any
+                                   Dmax); the layout query rejects a pair that does not fit         */
     int32_t budget;             /* nn_budget: gallery vectors kept per track (nn_matching.py:150);
                                    0 = None: unbounded, what deepdish.py:515-516 always passes      */
     int32_t feat_dim;           /* must be DD_FEAT_DIM                                              */

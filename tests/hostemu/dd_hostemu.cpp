@@ -17,6 +17,9 @@ int ddh_tracker_layout_query(const dd_tracker_config* cfg, dd_tracker_layout* ou
     return dd_layout_compute(cfg, out);
 }
 
+// shared memory of the matching step for T slots and D detections (what the layout check compares with the limit)
+long long ddh_match_smem_bytes(int T, int D) { return (long long)dd_match_smem_bytes(T, D, dd_set_table_slots(T)); }
+
 int ddh_tracker_init(void* state, const dd_tracker_config* cfg) {
     DDView V;
     int rc = dd_make_view(state, cfg, &V);

@@ -34,12 +34,15 @@ KNOBS = {
 }
 
 
-def _history(impl, S, nobj, dmax, tmax, budget, frames, seed, feat_noise, big_boxes=False):
-    """impl: "exact" (the f32 pass) or a KNOBS key (the half pre-pass with those knobs)."""
+def _history(impl, S, nobj, dmax, tmax, budget, frames, seed, feat_noise, big_boxes=False, scene=None, flags=0,
+             pool_fraction=0.5):
+    """impl: "exact" (the f32 pass) or a KNOBS key (the half pre-pass with those knobs).  scene: a factory of the
+    scene to run instead of Scene(S, nobj, dmax, ...); flags: the status the run must end with (0: bt.check())."""
     from deepdish_b200.batched import BatchedTracker
     knobs = dict(gallery_impl="exact") if impl == "exact" else KNOBS[impl]
-    bt = BatchedTracker(S, LABELS3, max_tracks=tmax, max_dets=dmax, budget=budget, max_age=30, page_cap=8, **knobs)
-    sc = Scene(S, nobj, dmax, n_labels=3, seed=seed, feat_noise=feat_noise)
+    bt = BatchedTracker(S, LABELS3, max_tracks=tmax, max_dets=dmax, budget=budget, max_age=30, page_cap=8,
+                        pool_fraction=pool_fraction, **knobs)
+    sc = scene() if scene is not None else Scene(S, nobj, dmax, n_labels=3, seed=seed, feat_noise=feat_noise)
     if big_boxes:                      # large slow boxes: many detections pass each track's Mahalanobis gate
         sc.size = sc.size * 4.0
         sc.vel = sc.vel * 0.2
@@ -52,7 +55,10 @@ def _history(impl, S, nobj, dmax, tmax, budget, frames, seed, feat_noise, big_bo
         cost = bt.v["cost"].cpu().numpy()
         state = bt.v["state"].cpu().numpy()
         out.append((ids, gate, cost, state, int(bt.v["work_ctl"][0])))
-    bt.check()
+    if flags:
+        assert bt.status() == flags
+    else:
+        bt.check()
     return out
 
 
